@@ -386,6 +386,26 @@ def time_runner(r, steps, warmup, sampler=None):
     return ms, kern_ms, launches
 
 
+def dump_outputs(r, d, budget=60 << 20):
+    """Writes what the last rollout returned to its caller (obs, rew, done, info: [T, E, ...]) as d/<name>.npy,
+    float32 (info: float64), for a fixed seeded sample of the envs that keeps the data within `budget` bytes;
+    d/env_ids.npy lists the sampled envs.  Engine seeds and actions are fixed, so the same arguments give the
+    same inputs on every run and two builds can be compared output for output."""
+    torch = r.torch
+    last = r.agather.buffers(r.k - 1) if r.agather is not None else (r.packed.rew, r.packed.done, r.packed.info)
+    outs = dict(zip(("obs", "rew", "done", "info"), (r.obs_buf,) + tuple(last)))
+    dtypes = {k: np.float64 if k == "info" else np.float32 for k in outs}
+    per_env = sum(x[:, 0].numel() * np.dtype(dtypes[k]).itemsize for k, x in outs.items())
+    n = max(1, min(r.E, budget // per_env))
+    ids = np.sort(np.random.RandomState(0).choice(r.E, n, replace=False))
+    idx = torch.as_tensor(ids, device=r.dev)
+    torch.cuda.synchronize()
+    os.makedirs(d, exist_ok=True)
+    for k, x in outs.items():
+        np.save(os.path.join(d, k + ".npy"), x.index_select(1, idx).cpu().numpy().astype(dtypes[k]))
+    np.save(os.path.join(d, "env_ids.npy"), ids.astype(np.float64))
+
+
 def roofline_of(wl, E, T, kern_ms):
     bpe = bytes_per_env_step(wl)
     peak, peak_kind = measured_peak_gbs()
@@ -523,7 +543,11 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the short runs of the other BASELINE configs")
     ap.add_argument("--exchange", default="overlap", choices=["overlap", "overlap-nccl", "nccl", "none"],
                     help="multi-GPU per-rollout exchange of rewards / dones / infos (see DESIGN.md 7)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed rollout (rank 0) as DIR/<name>.npy, at most 64 MB")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -584,6 +608,8 @@ def main():
     ms, kern_ms, launches = time_runner(r, a.steps, warmup, sampler)
     if sampler:
         sampler.join(timeout=2)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(r, a.dump_outputs)
     agent_steps_per_step = world * E * WL["agents"] * T * LAUNCHES_PER_STEP
     value = agent_steps_per_step * a.steps / (ms * 1e-3)
     mode, note, completion = r.mode, r.note, getattr(r, "completion", None)

@@ -6,8 +6,8 @@
   * ``pursuit_action_table`` the same decision tabulated per window cell (what the CUDA host code builds)
   * ``policy_draw``          the injected stream that stands in for ``action_space.sample()``
 
-Pinned: ``tests/test_heuristics.py`` (marker ``reference``) runs the real classes, loaded from
-/root/reference through ``oracle/refshim.load_reference_heuristics``, on the same inputs.
+Pinned: ``tests/test_heuristics.py`` compares it with the actions the real classes (loaded through
+``oracle/refshim.load_reference_heuristics``) took on the same inputs, recorded in ``tests/golden/ref_heuristics_*.npz``.
 """
 import math
 

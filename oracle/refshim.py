@@ -11,10 +11,9 @@ imports in ``sys.modules`` and puts the reference root on ``sys.path`` so that
     madrl_environments.pursuit.pursuit_evade.PursuitEvade
     madrl_environments.hostage.ContinuousHostageWorld
 
-can be imported and executed UNMODIFIED.  No reference file is copied or edited.  The reference
-only exists in the build container, so everything that uses this shim (``oracle/make_golden.py``
-and the ``reference``-marked tests) is skipped automatically when ``/root/reference`` is absent
-(e.g. on the GPU box); what travels are the golden vectors it produced (``tests/golden``).
+can be imported and executed UNMODIFIED.  No reference file is copied or edited.  Only recording
+uses this shim (``oracle/make_golden.py`` and ``MADRL_RECORD_REFERENCE=1`` runs of the tests,
+tests/reference_record.py); the tests compare with the golden vectors it produced (``tests/golden``).
 
 Stub behaviour follows the originals:
   * ``rltools.util.EzPickle``      -- pickle by constructor args (rltools/rltools/util.py:261-288)

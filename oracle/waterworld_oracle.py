@@ -3,7 +3,8 @@
 This is a restatement -- not a copy -- of the algorithm in the reference file
 ``madrl_environments/pursuit/waterworld.py`` (cited per function below, ``ww:LINE``).  State is
 held as plain arrays instead of ``Archea`` objects.  It is pinned against the real reference
-classes (imported through ``oracle/refshim.py``) by ``tests/test_waterworld_oracle.py`` (marker ``reference``) and by
+classes (imported through ``oracle/refshim.py``; their runs recorded in ``tests/golden/ref_ww_oracle_*.npz``) by
+``tests/test_waterworld_oracle.py`` and by
 the golden vectors in ``tests/golden`` produced by ``oracle/make_golden.py``; on identical
 injected random streams the two agree bit for bit in float64.
 

@@ -2,7 +2,7 @@
 kernels (madrl_ww_rollout_heuristic / madrl_pursuit_rollout_heuristic):
 
   * the oracle restatement (oracle/heuristics_oracle.py) is pinned to the REAL classes
-    (heuristics/waterworld.py, heuristics/pursuit.py, loaded through the shim; marker `reference`);
+    (heuristics/waterworld.py, heuristics/pursuit.py; their actions recorded, tests/reference_record.py);
   * the kernel source, run on the CPU by the warp emulator (tests/emu), closes the loop exactly as the
     oracle policy driving the oracle env does.  The same checks run on the GPU in
     tests/test_heuristics_gpu.py.
@@ -20,8 +20,8 @@ from oracle.heuristics_oracle import (pursuit_action, pursuit_action_table, poli
 from oracle.philox import Stream
 from oracle.pursuit_oracle import PursuitOracle
 from oracle.waterworld_oracle import WaterworldOracle
+from reference_record import recorded
 
-needs_ref = pytest.mark.skipif(not refshim.reference_available(), reason="reference tree not present")
 needs_cxx = pytest.mark.skipif(shutil.which(os.environ.get("CXX", "g++")) is None, reason="no host C++ compiler")
 
 
@@ -30,12 +30,10 @@ def f32(x):
 
 
 # ------------------------------------------------------------------------------ oracle == reference
-@needs_ref
-@pytest.mark.reference
 def test_waterworld_policy_oracle_equals_reference_bitwise():
-    W, _, _ = refshim.load_reference_heuristics()
-    pol = W(None, None)
+    """The reference policy's actions (recorded) on 600 random observations, bit for bit."""
     rs = np.random.RandomState(0)
+    cases = []
     for K in (30, 7):
         D = 7 * K + 3
         for i in range(300):
@@ -43,8 +41,14 @@ def test_waterworld_policy_oracle_equals_reference_bitwise():
             o[7 * K:7 * K + 2] = rs.rand(2) < 0.3
             if i == 5:
                 o[:] = 0
-            a, _ = pol.sample_actions(o[None])
-            assert np.array_equal(a[0], waterworld_action(o)), (K, i)
+            cases.append((K, i, o))
+
+    def reference():
+        pol = refshim.load_reference_heuristics()[0](None, None)
+        return dict(actions=np.array([pol.sample_actions(o[None])[0][0] for _, _, o in cases]))
+    ref = recorded("heuristics_waterworld", reference)["actions"]
+    for (K, i, o), a in zip(cases, ref):
+        assert np.array_equal(a, waterworld_action(o)), (K, i)
 
 
 class _Space(object):
@@ -55,32 +59,37 @@ class _Space(object):
         return self.draws.pop(0)
 
 
-@needs_ref
-@pytest.mark.reference
 @pytest.mark.parametrize("py2", [False, True])
 def test_pursuit_policy_oracle_equals_reference(py2):
     """py2=False: heuristics/pursuit.py executed as is (Python 3: `xs / 2` is a true division).
-    py2=True: the same source with line 23's two divisions spelt `//`, what they mean in Python 2."""
-    _, P, src = refshim.load_reference_heuristics()
-    if py2:
-        ported = src.replace("x, y = xs / 2, ys / 2", "x, y = xs // 2, ys // 2")
-        assert ported != src
-        mod = types.ModuleType("_ref_heuristics_pursuit_py2")
-        exec(compile(ported.split("if __name__")[0], "heuristics/pursuit.py[py2 division]", "exec"), mod.__dict__)
-        P = mod.PursuitHeuristicPolicy
+    py2=True: the same source with line 23's two divisions spelt `//`, what they mean in Python 2.
+    The reference policy's actions on 1600 random windows are recorded; 77 stands for a sampled action."""
     rs = np.random.RandomState(1)
+    cases = []
     for R in (7, 4, 5, 9):
-        tab = pursuit_action_table(R, py2)
         for i in range(400):
             o = np.zeros((R, R, 4))
             o[..., 2] = (rs.rand(R, R) < 0.06) * 0.1
-            a, _ = P(None, _Space([77])).sample_actions(o)
-            assert a == pursuit_action(o, lambda: 77, py2), (R, i)
-            if a != 77:   # the tabulated form the CUDA host code uses
-                xev, yev = np.nonzero(o[..., 2])
-                c = float(R // 2) if py2 else R / 2
-                k = np.argmin((xev - c) ** 2 + (yev - c) ** 2)
-                assert tab[xev[k] * R + yev[k]] == a
+            cases.append((R, i, o))
+
+    def reference():
+        _, P, src = refshim.load_reference_heuristics()
+        if py2:
+            ported = src.replace("x, y = xs / 2, ys / 2", "x, y = xs // 2, ys // 2")
+            assert ported != src
+            mod = types.ModuleType("_ref_heuristics_pursuit_py2")
+            exec(compile(ported.split("if __name__")[0], "heuristics/pursuit.py[py2 division]", "exec"), mod.__dict__)
+            P = mod.PursuitHeuristicPolicy
+        return dict(actions=np.array([P(None, _Space([77])).sample_actions(o)[0] for _, _, o in cases]))
+    ref = recorded("heuristics_pursuit_py%d" % (2 if py2 else 3), reference)["actions"]
+    tabs = {R: pursuit_action_table(R, py2) for R in (7, 4, 5, 9)}
+    for (R, i, o), a in zip(cases, ref):
+        assert a == pursuit_action(o, lambda: 77, py2), (R, i)
+        if a != 77:   # the tabulated form the CUDA host code uses
+            xev, yev = np.nonzero(o[..., 2])
+            c = float(R // 2) if py2 else R / 2
+            k = np.argmin((xev - c) ** 2 + (yev - c) ** 2)
+            assert tabs[R][xev[k] * R + yev[k]] == a
 
 
 # ------------------------------------------------------------------------------ emulated kernels

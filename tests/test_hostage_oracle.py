@@ -1,5 +1,5 @@
 """Pin the ContinuousHostageWorld oracle against golden vectors recorded from the real reference
-and, where the reference tree exists, against the reference classes themselves."""
+and against long runs of the reference classes themselves (their side recorded, tests/reference_record.py)."""
 import json
 import os
 
@@ -9,6 +9,7 @@ import pytest
 from conftest import GOLDEN_DIR
 from oracle.hostage_oracle import HostageOracle
 from oracle.philox import Stream
+from reference_record import assert_same_trace, recorded, trace
 
 HW_GOLDEN = ["hw_c5", "hw_c5_local", "hw_dense", "hw_k12"]
 
@@ -38,7 +39,6 @@ def test_oracle_reproduces_golden(name):
     assert o.np_random.counter == int(g["counter"])
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("args,kw,steps,seed,std", [
     ((10, 16, 16, 4, 2), {}, 700, 1, 0.5),
     ((10, 16, 16, 4, 2), dict(reward_mech='local'), 700, 2, 2.0),
@@ -46,22 +46,19 @@ def test_oracle_reproduces_golden(name):
     ((4, 6, 8, 2, 1), dict(radius=0.04, n_sensors=12, key_radius=0.05, bomb_radius=0.02), 1500, 4, 3.0),
 ])
 def test_oracle_equals_reference_bitwise(args, kw, steps, seed, std):
-    from oracle.refshim import load_reference
-    HW = load_reference()[2]
-    ref = HW(*args, **kw)
-    ref.np_random = Stream(seed, 3)
-    orc = HostageOracle(*args, rng=Stream(seed, 3), **kw)
-    assert all(np.array_equal(a, b) for a, b in zip(ref.reset(), orc.reset()))
+    """The oracle and the reference class, same stream and actions: every observation, reward, done, info and
+    reset identical and the same number of draws (reference side recorded)."""
     ar = np.random.RandomState(seed)
-    for t in range(steps):
-        a = ar.randn(args[0] * 2) * std
-        o1, r1, d1, i1 = ref.step(a)
-        o2, r2, d2, i2 = orc.step(a)
-        assert all(np.array_equal(x, y) for x, y in zip(o1, o2)), t
-        assert np.array_equal(r1, r2) and d1 == d2 and i1 == i2, t
-        if d1:
-            assert all(np.array_equal(a_, b_) for a_, b_ in zip(ref.reset(), orc.reset()))
-    assert ref.np_random.counter == orc.np_random.counter
+    actions = [ar.randn(args[0] * 2) * std for _ in range(steps)]
+
+    def reference():
+        from oracle.refshim import load_reference
+        ref = load_reference()[2](*args, **kw)
+        ref.np_random = Stream(seed, 3)
+        return dict(trace(ref, actions), counter=ref.np_random.counter)
+    orc = HostageOracle(*args, rng=Stream(seed, 3), **kw)
+    got = dict(trace(orc, actions), counter=orc.np_random.counter)
+    assert_same_trace(got, recorded("hw_oracle_s%d" % seed, reference))
 
 
 def test_scripted_quirks():

@@ -1,10 +1,11 @@
-"""Post-processing passes: oracle vs the REAL reference wrappers (CPU, needs /root/reference) and
-CUDA kernels vs oracle (GPU)."""
+"""Post-processing passes: oracle vs the REAL reference wrappers (CPU; their outputs recorded,
+tests/reference_record.py) and CUDA kernels vs oracle (GPU)."""
 import numpy as np
 import pytest
 
 from oracle import postproc_oracle as po
 from oracle.postproc_oracle import StandardizeEnv, discount_cumsum, episode_stats_env, frame_stack_env, gae_env
+from reference_record import digest, recorded
 
 
 class ScriptedEnv(object):
@@ -32,85 +33,107 @@ class ScriptedEnv(object):
         return [x.copy() for x in o], list(r), False, {}
 
 
-@pytest.mark.reference
 def test_oracles_equal_reference_wrappers():
-    from oracle.refshim import install
-    install()
-    import gym.spaces as spaces
-    import madrl_environments as me
-    me.ent = None  # noqa  (ObservationBuffer.agents has a typo'd name; not used here)
+    """ObservationBuffer and StandardizedEnv of the reference around a scripted env, against the oracle's
+    frame stack and standardiser, bit for bit (reference side recorded)."""
     rs = np.random.RandomState(0)
     T, A, D, B = 40, 3, 5, 4
     obs0, obs, rew = rs.randn(A, D), rs.randn(T, A, D), rs.randn(T, A)
+
+    def reference():
+        from oracle.refshim import install
+        install()
+        import gym.spaces as spaces
+        import madrl_environments as me
+        me.ent = None  # noqa  (ObservationBuffer.agents has a typo'd name; not used here)
+        w = me.ObservationBuffer.__new__(me.ObservationBuffer)
+        w._unwrapped = ScriptedEnv(obs0, obs, rew, spaces)
+        w._buffer_size = B
+        w._buffer = [np.zeros((D, B)) for _ in range(A)]
+        out = dict(buffer0=np.array(w.reset()), buffer=np.array([np.array(w.step(None)[0]) for _ in range(T)]))
+        s = me.StandardizedEnv(ScriptedEnv(obs0, obs, rew, spaces), scale_reward=0.5, enable_obsnorm=True,
+                               enable_rewnorm=True, obs_alpha=0.05, rew_alpha=0.02)
+        out["std0"] = np.array(s.reset())
+        steps = [s.step(None) for _ in range(T)]
+        return dict(out, std_obs=np.array([np.array(x[0]) for x in steps]),
+                    std_rew=np.array([np.array(x[1]) for x in steps]))
+    ref = recorded("postproc_wrappers", reference)
     # ObservationBuffer
-    w = me.ObservationBuffer.__new__(me.ObservationBuffer)
-    w._unwrapped = ScriptedEnv(obs0, obs, rew, spaces)
-    w._buffer_size = B
-    w._buffer = [np.zeros((D, B)) for _ in range(A)]
-    out0 = np.array(w.reset())
-    ref = np.array([np.array(w.step(None)[0]) for _ in range(T)])
     o0, o = frame_stack_env(obs0, obs, np.zeros(T, bool), B)
-    assert np.array_equal(out0, o0) and np.array_equal(ref, o)
+    assert np.array_equal(ref["buffer0"], o0) and np.array_equal(ref["buffer"], o)
     # StandardizedEnv
-    env = ScriptedEnv(obs0, obs, rew, spaces)
-    s = me.StandardizedEnv(env, scale_reward=0.5, enable_obsnorm=True, enable_rewnorm=True,
-                           obs_alpha=0.05, rew_alpha=0.02)
     mine = StandardizeEnv(A, D, 0.5, True, True, 0.05, 0.02)
-    assert np.array_equal(np.array(s.reset()), mine.obs(obs0))
+    assert np.array_equal(ref["std0"], mine.obs(obs0))
     for t in range(T):
-        so, sr, _, _ = s.step(None)
-        assert np.array_equal(np.array(so), mine.obs(obs[t]))
-        assert np.array_equal(np.array(sr), mine.rew(rew[t]))
+        assert np.array_equal(ref["std_obs"][t], mine.obs(obs[t]))
+        assert np.array_equal(ref["std_rew"][t], mine.rew(rew[t]))
 
 
-@pytest.mark.reference
 def test_episode_stats_oracle_equals_reference_wrapper():
-    from oracle.refshim import install
-    install()
-    import gym.spaces as spaces
-    import madrl_environments as me
+    """The episode statistics DiagnosticsWrapper logs, against the oracle's (reference side recorded)."""
     rs = np.random.RandomState(3)
     T, A, D = 60, 3, 2
     obs0, obs, rew = rs.randn(A, D), rs.randn(T, A, D), rs.randn(T, A)
     done = np.zeros(T, bool)
     done[[7, 30]] = True
 
-    class Env(ScriptedEnv):
-        def step(self, a):
-            o, r, _, i = ScriptedEnv.step(self, a)
-            return o, np.asarray(r), bool(done[self.t - 1]), i
-    w = me.DiagnosticsWrapper(Env(obs0, obs, rew, spaces), discount=0.9, max_traj_len=12, log_interval=10 ** 9)
-    w.reset()
-    got = []
-    for t in range(T):
-        _, _, _, log = w.step(None)
-        if 'global/episode_length' in log:
-            got.append((t, np.array([log['global/episode_reward_agent%d' % a] for a in range(A)]),
-                        log['global/episode_avg_reward'], log['global/episode_disc_return'],
-                        log['global/episode_length']))
+    def reference():
+        from oracle.refshim import install
+        install()
+        import gym.spaces as spaces
+        import madrl_environments as me
+
+        class Env(ScriptedEnv):
+            def step(self, a):
+                o, r, _, i = ScriptedEnv.step(self, a)
+                return o, np.asarray(r), bool(done[self.t - 1]), i
+        w = me.DiagnosticsWrapper(Env(obs0, obs, rew, spaces), discount=0.9, max_traj_len=12, log_interval=10 ** 9)
+        w.reset()
+        got = []
+        for t in range(T):
+            _, _, _, log = w.step(None)
+            if 'global/episode_length' in log:
+                got.append((t, [log['global/episode_reward_agent%d' % a] for a in range(A)],
+                            log['global/episode_avg_reward'], log['global/episode_disc_return'],
+                            log['global/episode_length']))
+        return {k: np.array([g[j] for g in got]) for j, k in enumerate(("t", "agent", "avg", "disc", "length"))}
+    ref = recorded("postproc_episode_stats", reference)
+    got = list(zip(*(ref[k] for k in ("t", "agent", "avg", "disc", "length"))))
     mine = episode_stats_env(rew, done, 0.9, 12)
     assert len(got) == len(mine) >= 5
     for g, m in zip(got, mine):
         assert g[0] == m[0] and np.array_equal(g[1], m[1]) and g[2] == m[2] and g[3] == m[3] and g[4] == m[4]
 
 
-@pytest.mark.reference
 def test_batch_statistics_oracle_equals_rllab_functions():
     """center_advantages / shift_advantages_to_positive / explained_variance_1d / discount_cumsum
     of the oracle against the reference's own functions (rllab/rllab/algos/util.py:7-12,
-    rllab/rllab/misc/special.py:51-59,107-111), bit for bit."""
-    from oracle.refshim import load_rllab_numeric
-    util, special = load_rllab_numeric()
+    rllab/rllab/misc/special.py:51-59,107-111), bit for bit (reference side recorded; arrays as digests)."""
     rs = np.random.RandomState(5)
-    for n in (1, 2, 17, 4096):
-        adv, y = rs.randn(n) * 3 + 1, rs.randn(n)
-        assert np.array_equal(po.center_advantages(adv), util.center_advantages(adv))
-        assert np.array_equal(po.shift_advantages_to_positive(adv), util.shift_advantages_to_positive(adv))
-        assert po.explained_variance_1d(adv, y) == special.explained_variance_1d(adv, y)
-        assert np.array_equal(discount_cumsum(adv, 0.97), special.discount_cumsum(adv, 0.97))
+    ns = (1, 2, 17, 4096)
+    inputs = [(rs.randn(n) * 3 + 1, rs.randn(n)) for n in ns]
     const = np.full(9, 2.5)
-    assert po.explained_variance_1d(const, const) == special.explained_variance_1d(const, const) == 1
-    assert po.explained_variance_1d(rs.randn(9), const) == special.explained_variance_1d(rs.randn(9), const) == 0
+    noise = rs.randn(9), rs.randn(9)
+
+    def reference():
+        from oracle.refshim import load_rllab_numeric
+        util, special = load_rllab_numeric()
+        out = {}
+        for n, (adv, y) in zip(ns, inputs):
+            out.update({"center%d" % n: digest(util.center_advantages(adv)),
+                        "shift%d" % n: digest(util.shift_advantages_to_positive(adv)),
+                        "ev%d" % n: special.explained_variance_1d(adv, y),
+                        "cumsum%d" % n: digest(special.discount_cumsum(adv, 0.97))})
+        return dict(out, ev_const=special.explained_variance_1d(const, const),
+                    ev_noise=special.explained_variance_1d(noise[1], const))
+    ref = recorded("postproc_batch_statistics", reference)
+    for n, (adv, y) in zip(ns, inputs):
+        assert np.array_equal(digest(po.center_advantages(adv)), ref["center%d" % n])
+        assert np.array_equal(digest(po.shift_advantages_to_positive(adv)), ref["shift%d" % n])
+        assert po.explained_variance_1d(adv, y) == ref["ev%d" % n]
+        assert np.array_equal(digest(discount_cumsum(adv, 0.97)), ref["cumsum%d" % n])
+    assert po.explained_variance_1d(const, const) == ref["ev_const"] == 1
+    assert po.explained_variance_1d(noise[0], const) == ref["ev_noise"] == 0
 
 
 def test_gae_oracle_matches_rllab_formulas():

@@ -1,5 +1,5 @@
-"""Pin the PursuitEvade oracle: golden vectors recorded from the real reference and, where the
-reference tree exists, live bit-exact differential runs."""
+"""Pin the PursuitEvade oracle: golden vectors recorded from the real reference and long bit-exact
+differential runs against it (its side recorded, tests/reference_record.py)."""
 import json
 import os
 
@@ -9,6 +9,7 @@ import pytest
 from conftest import GOLDEN_DIR, ROOT
 from oracle.philox import Stream
 from oracle.pursuit_oracle import PursuitOracle
+from reference_record import assert_same_trace, recorded, trace
 
 PE_GOLDEN = ["pe_c3", "pe_c3_global", "pe_ncatch", "pe_window", "pe_small", "pe_even_range", "pe_crowd", "pe_random_opp"]
 
@@ -50,7 +51,6 @@ def test_oracle_reproduces_golden(name):
     assert o.rng.counter == int(g["counter"])
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("kw,steps,seed,small", [
     (dict(n_evaders=30, n_pursuers=8, obs_range=7, surround=True, n_catch=2, flatten=True,
           reward_mech='local', catchr=0.1, term_pursuit=5.0, sample_maps=True, include_id=True), 500, 1, False),
@@ -64,21 +64,21 @@ def test_oracle_reproduces_golden(name):
           random_opponents=True, max_opponents=6), 600, 8, True),
 ])
 def test_oracle_equals_reference_bitwise(kw, steps, seed, small):
-    from oracle.refshim import make_reference_pursuit
+    """The oracle and the reference class, same stream and actions, reset after a done step and every 97 steps:
+    every observation, reward, done, info and reset identical and the same number of draws (reference side
+    recorded)."""
     maps = small_map() if small else np.load(os.path.join(ROOT, "maps", "map_pool16.npy"))
-    ref = make_reference_pursuit(maps, Stream(seed, 5), **kw)
-    orc = PursuitOracle(maps, rng=Stream(seed, 5), **kw)
-    assert all(np.array_equal(a, b) for a, b in zip(ref.reset(), orc.reset()))
     ar = np.random.RandomState(seed)
-    for t in range(steps):
-        a = ar.randint(0, 5, size=kw['n_pursuers'])
-        o1, r1, d1, i1 = ref.step(a)
-        o2, r2, d2, i2 = orc.step(a)
-        assert all(np.array_equal(x, y) for x, y in zip(o1, o2)), t
-        assert np.array_equal(np.asarray(r1), np.asarray(r2)) and d1 == d2 and i1 == i2, t
-        if d1 or t % 97 == 96:
-            assert all(np.array_equal(a_, b_) for a_, b_ in zip(ref.reset(), orc.reset()))
-    assert ref.evader_controller.rng.counter == orc.rng.counter
+    actions = [ar.randint(0, 5, size=kw['n_pursuers']) for _ in range(steps)]
+    every97 = lambda t: t % 97 == 96                                       # noqa: E731
+
+    def reference():
+        from oracle.refshim import make_reference_pursuit
+        ref = make_reference_pursuit(maps, Stream(seed, 5), **kw)
+        return dict(trace(ref, actions, every97), counter=ref.evader_controller.rng.counter)
+    orc = PursuitOracle(maps, rng=Stream(seed, 5), **kw)
+    got = dict(trace(orc, actions, every97), counter=orc.rng.counter)
+    assert_same_trace(got, recorded("pe_oracle_s%d" % seed, reference))
 
 
 def test_scripted_quirks():

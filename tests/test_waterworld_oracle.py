@@ -1,5 +1,5 @@
-"""Pin the Waterworld oracle: golden vectors (from the real reference) and, where the reference
-tree exists, live differential runs against the reference classes themselves."""
+"""Pin the Waterworld oracle: golden vectors (from the real reference) and long differential runs
+against the reference classes themselves (their side recorded, tests/reference_record.py)."""
 import json
 import os
 
@@ -8,6 +8,7 @@ import pytest
 
 from conftest import GOLDEN_DIR
 from oracle.philox import Stream
+from reference_record import assert_same_trace, recorded, trace
 from oracle.waterworld_oracle import WaterworldOracle
 
 WW_GOLDEN = ["ww_c2", "ww_dense", "ww_c4", "ww_global_nospeed"]
@@ -37,7 +38,6 @@ def test_oracle_reproduces_golden(name):
     assert o.np_random.counter == int(g["counter"])
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("cfg,steps,seed", [
     (dict(n_pursuers=5, n_evaders=5), 1200, 1),
     (dict(n_pursuers=5, n_evaders=5, n_coop=1, obstacle_loc=None, reward_mech='global'), 1100, 2),
@@ -46,23 +46,20 @@ def test_oracle_reproduces_golden(name):
           n_coop=1, radius=0.05), 1100, 4),
 ])
 def test_oracle_equals_reference_bitwise(cfg, steps, seed):
-    from oracle.refshim import load_reference
-    MAWaterWorld = load_reference()[0]
-    ref = MAWaterWorld(**cfg)
-    ref.np_random = Stream(seed, 7)
-    orc = WaterworldOracle(rng=Stream(seed, 7), **cfg)
-    assert all(np.array_equal(a, b) for a, b in zip(ref.reset(), orc.reset()))
+    """The oracle and the reference class, same stream and actions: every observation, reward, done, info and
+    reset identical, the same number of draws, the same final evader positions (reference side recorded)."""
     ar = np.random.RandomState(seed)
-    for t in range(steps):
-        a = ar.randn(cfg['n_pursuers'] * 2) * 0.5
-        o1, r1, d1, i1 = ref.step(a)
-        o2, r2, d2, i2 = orc.step(a)
-        assert all(np.array_equal(x, y) for x, y in zip(o1, o2)), t
-        assert np.array_equal(r1, r2) and d1 == d2 and i1 == i2, t
-        if d1:
-            assert all(np.array_equal(a_, b_) for a_, b_ in zip(ref.reset(), orc.reset()))
-    assert ref.np_random.counter == orc.np_random.counter
-    assert np.array_equal(np.array([p.position for p in ref._evaders]), orc.ex)
+    actions = [ar.randn(cfg['n_pursuers'] * 2) * 0.5 for _ in range(steps)]
+
+    def reference():
+        from oracle.refshim import load_reference
+        ref = load_reference()[0](**cfg)
+        ref.np_random = Stream(seed, 7)
+        return dict(trace(ref, actions), counter=ref.np_random.counter,
+                    final_ex=np.array([p.position for p in ref._evaders]))
+    orc = WaterworldOracle(rng=Stream(seed, 7), **cfg)
+    got = dict(trace(orc, actions), counter=orc.np_random.counter, final_ex=orc.ex)
+    assert_same_trace(got, recorded("ww_oracle_s%d" % seed, reference))
 
 
 def test_reset_consumes_one_step_and_quirks():
