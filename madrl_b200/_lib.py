@@ -102,22 +102,6 @@ def _declare(lib):
     lib.madrl_copy_async.argtypes = [vp, vp, C.c_size_t, vp]
     lib.madrl_stream_write32.argtypes = [vp, vp, C.c_uint32]
     lib.madrl_stream_wait_geq32.argtypes = [vp, vp, C.c_uint32]
-    lib.madrl_ww_state_layout.argtypes = [C.POINTER(WWConfig), C.POINTER(WWLayout)]
-    lib.madrl_ww_create.argtypes = [C.POINTER(WWConfig), vp, C.POINTER(vp)]
-    lib.madrl_ww_destroy.argtypes = [vp]
-    lib.madrl_ww_state_ptr.argtypes = [vp]
-    lib.madrl_ww_state_ptr.restype = vp
-    lib.madrl_ww_seed.argtypes = [vp, u64, vp]
-    lib.madrl_ww_set_launch.argtypes = [vp, i32, i32]
-    lib.madrl_ww_set_terminal_obs.argtypes = [vp, vp]
-    lib.madrl_ww_set_peers.argtypes = [vp, i32, i32, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
-    lib.madrl_ww_reset.argtypes = [vp, vp, vp, vp]
-    lib.madrl_ww_rollout.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, vp]
-    lib.madrl_ww_rollout_heuristic.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, i32, vp]
-    lib.madrl_ww_step.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp]
-    lib.madrl_ww_reset_host.argtypes = [vp, vp, vp]
-    lib.madrl_ww_rollout_host.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32]
-    lib.madrl_ww_rollout_host2.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, i32]
     lib.madrl_ww_heuristic_actions.argtypes = [i32, C.c_size_t, i32, i32, vp, vp, vp]
     lib.madrl_pursuit_heuristic_actions.argtypes = [C.c_size_t, i32, i32, i32, i32, vp, vp, vp, vp, vp]
     lib.madrl_gae_f32.argtypes = [i32, i32, i32, vp, vp, vp, vp, C.c_double, C.c_double, vp, vp, vp]
@@ -130,36 +114,28 @@ def _declare(lib):
     lib.madrl_paths_pack_u32.argtypes = [i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]
     lib.madrl_moments_f32.argtypes = [C.c_size_t, vp, vp, vp, vp, vp]
     lib.madrl_center_advantages_f32.argtypes = [C.c_size_t, vp, i32, i32, vp, vp, vp]
-    lib.madrl_hostage_state_layout.argtypes = [C.POINTER(HWConfig), C.POINTER(HWLayout)]
-    lib.madrl_hostage_create.argtypes = [C.POINTER(HWConfig), vp, C.POINTER(vp)]
-    lib.madrl_hostage_destroy.argtypes = [vp]
-    lib.madrl_hostage_state_ptr.argtypes = [vp]
-    lib.madrl_hostage_state_ptr.restype = vp
-    lib.madrl_hostage_seed.argtypes = [vp, u64, vp]
-    lib.madrl_hostage_set_launch.argtypes = [vp, i32, i32]
-    lib.madrl_hostage_set_terminal_obs.argtypes = [vp, vp]
-    lib.madrl_hostage_reset.argtypes = [vp, vp, vp, vp]
-    lib.madrl_hostage_rollout.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, vp]
-    lib.madrl_hostage_step.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp]
-    lib.madrl_hostage_reset_host.argtypes = [vp, vp, vp]
-    lib.madrl_hostage_rollout_host.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32]
-    lib.madrl_hostage_rollout_host2.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, i32]
-    lib.madrl_pursuit_state_layout.argtypes = [C.POINTER(PEConfig), C.POINTER(PELayout)]
-    lib.madrl_pursuit_create.argtypes = [C.POINTER(PEConfig), vp, vp, C.POINTER(vp)]
-    lib.madrl_pursuit_destroy.argtypes = [vp]
-    lib.madrl_pursuit_state_ptr.argtypes = [vp]
-    lib.madrl_pursuit_state_ptr.restype = vp
-    lib.madrl_pursuit_seed.argtypes = [vp, u64, vp]
-    lib.madrl_pursuit_set_launch.argtypes = [vp, i32, i32]
-    lib.madrl_pursuit_set_terminal_obs.argtypes = [vp, vp]
+    for fam, cfg, lay in (("ww", WWConfig, WWLayout), ("pursuit", PEConfig, PELayout),
+                          ("hostage", HWConfig, HWLayout)):
+        f = lambda name: getattr(lib, "madrl_%s_%s" % (fam, name))   # noqa: E731
+        f("state_layout").argtypes = [C.POINTER(cfg), C.POINTER(lay)]
+        f("create").argtypes = [C.POINTER(cfg), vp, C.POINTER(vp)]
+        f("destroy").argtypes = [vp]
+        f("state_ptr").argtypes = [vp]
+        f("state_ptr").restype = vp
+        f("seed").argtypes = [vp, u64, vp]
+        f("set_launch").argtypes = [vp, i32, i32]
+        f("set_terminal_obs").argtypes = [vp, vp]
+        f("reset").argtypes = [vp, vp, vp, vp]
+        f("rollout").argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, vp]
+        f("step").argtypes = [vp, vp, vp, vp, vp, vp, i32, vp]
+        f("reset_host").argtypes = [vp, vp, vp]
+        f("rollout_host").argtypes = [vp, i32, vp, vp, vp, vp, vp, i32]
+        f("rollout_host2").argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, i32]
+    lib.madrl_pursuit_create.argtypes = [C.POINTER(PEConfig), vp, vp, C.POINTER(vp)]   # + the map pool
     lib.madrl_pursuit_set_params.argtypes = [vp, C.c_double, C.c_double]
-    lib.madrl_pursuit_reset.argtypes = [vp, vp, vp, vp]
-    lib.madrl_pursuit_rollout.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, vp]
+    lib.madrl_ww_set_peers.argtypes = [vp, i32, i32, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
+    lib.madrl_ww_rollout_heuristic.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, i32, vp]
     lib.madrl_pursuit_rollout_heuristic.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, i32, i32, vp]
-    lib.madrl_pursuit_step.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp]
-    lib.madrl_pursuit_reset_host.argtypes = [vp, vp, vp]
-    lib.madrl_pursuit_rollout_host.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32]
-    lib.madrl_pursuit_rollout_host2.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, i32]
 
 
 def lib():
@@ -192,13 +168,14 @@ def lib():
 def require_tensor(t, name, dtype, shape, device):
     """Validate a caller-supplied tensor before its data_ptr() crosses the C ABI (a wrong dtype,
     a non-contiguous view or a short buffer would otherwise be silent garbage or an out-of-bounds
-    device write).  `device`: a torch.device for device buffers, 'cpu' for host buffers."""
+    device write).  `shape` None: any shape.  `device`: a torch.device for device buffers, 'cpu' for
+    host buffers."""
     import torch
     if not isinstance(t, torch.Tensor):
         raise TypeError("%s must be a torch.Tensor, got %r" % (name, type(t)))
     if t.dtype != dtype:
         raise TypeError("%s must be %s, got %s" % (name, dtype, t.dtype))
-    if tuple(t.shape) != tuple(shape):
+    if shape is not None and tuple(t.shape) != tuple(shape):
         raise ValueError("%s must have shape %s, got %s" % (name, tuple(shape), tuple(t.shape)))
     if not t.is_contiguous():
         raise ValueError("%s must be contiguous" % name)

@@ -1,8 +1,11 @@
-// Library-wide host helpers: error string, launch counter, device queries.
+// Library-wide host helpers: error string, launch counter, device queries, the env handle core.
+#include <math.h>
 #include <stdarg.h>
 #include <string.h>
+#include <new>
 
 #include "common.cuh"
+#include "host_pipeline.cuh"
 
 namespace madrl {
 
@@ -25,6 +28,71 @@ int sm_count(int device) {
     return -1;
   }
   return n;
+}
+
+// ---- handle core (host_pipeline.cuh) ------------------------------------------------------------
+int core_init(EnvCore* h, void* state_dev, size_t total_bytes) {
+  cudaError_t e = cudaGetDevice(&h->device);
+  if (e != cudaSuccess) { set_error("cudaGetDevice: %s", cudaGetErrorString(e)); return MADRL_ECUDA; }
+  h->sms = sm_count(h->device);
+  if (h->sms <= 0) return MADRL_ECUDA;
+  if (state_dev) {
+    h->state = (char*)state_dev;
+  } else {
+    char* p = nullptr;
+    e = cudaMalloc((void**)&p, total_bytes);
+    if (e != cudaSuccess) { set_error("cudaMalloc(%zu): %s", total_bytes, cudaGetErrorString(e)); return MADRL_ENOMEM; }
+    h->state = p;
+    h->owns_state = true;
+  }
+  e = cudaMemset(h->state, 0, total_bytes);
+  if (e != cudaSuccess) { set_error("cudaMemset: %s", cudaGetErrorString(e)); return MADRL_ECUDA; }
+  return MADRL_OK;
+}
+
+void core_release(EnvCore* h) {
+  if (h->owns_state && h->state) cudaFree(h->state);
+  h->pipe.destroy();
+}
+
+int core_clear_counters(EnvCore* h, size_t rng_counter_off, int n_envs, void* stream) {
+  MADRL_CUDA_CHECK(cudaMemsetAsync(h->state + rng_counter_off, 0, 8 * (size_t)n_envs, (cudaStream_t)stream));
+  return MADRL_OK;
+}
+
+int core_set_terminal_obs(EnvCore* h, void* term_obs_dev) {
+  MADRL_REQUIRE(h != nullptr, "handle is NULL");
+  h->term_obs = term_obs_dev;
+  return MADRL_OK;
+}
+
+int core_set_launch(EnvCore* h, int warps_per_block, int blocks_per_sm) {
+  MADRL_REQUIRE(h != nullptr, "handle is NULL");
+  // warps_per_block is ignored (blocks are one warp) but still range-checked: the ABI has always refused > 4
+  MADRL_REQUIRE(warps_per_block >= 0 && warps_per_block <= 4, "warps_per_block must be in [0,4]");
+  MADRL_REQUIRE(blocks_per_sm >= 0 && blocks_per_sm <= 32, "blocks_per_sm must be in [0,32]");
+  h->blocks_per_sm = blocks_per_sm;
+  return MADRL_OK;
+}
+
+template <typename real>
+static int upload_sensor_table_t(char* dst_dev, int K) {
+  real* tab = new (std::nothrow) real[2 * (size_t)K];
+  if (!tab) return MADRL_ENOMEM;
+  const double step = (2.0 * M_PI - 0.0) / (double)K;
+  for (int k = 0; k < K; ++k) {
+    const double a = (double)k * step + 0.0;
+    tab[k] = (real)cos(a);
+    tab[K + k] = (real)sin(a);
+  }
+  cudaError_t e = cudaMemcpy(dst_dev, tab, sizeof(real) * 2 * K, cudaMemcpyHostToDevice);
+  delete[] tab;
+  MADRL_CUDA_CHECK(e);
+  return MADRL_OK;
+}
+
+int upload_sensor_table(char* dst_dev, int K, bool fp64) {
+  return fp64 ? upload_sensor_table_t<double>(dst_dev, K) : upload_sensor_table_t<float>(dst_dev, K);
 }
 
 }  // namespace madrl

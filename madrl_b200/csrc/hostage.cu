@@ -429,15 +429,9 @@ hw_kernel(const __grid_constant__ HWParams<real> p) {
 // =================================================================================================
 using namespace madrl;
 
-struct madrl_hostage {
+struct madrl_hostage : EnvCore {
   madrl_hostage_config cfg;
   madrl_hostage_layout lay;
-  char* state;
-  bool owns_state;
-  int device, sms;
-  int warps_per_block, blocks_per_sm;
-  madrl::HostPipe pipe;   // staging + streams of the host-buffer entry points (lazily created)
-  void* term_obs;         // madrl_hostage_set_terminal_obs (NULL = off)
 };
 
 static int hw_validate(const madrl_hostage_config* c) {
@@ -476,23 +470,6 @@ extern "C" int madrl_hostage_state_layout(const madrl_hostage_config* c, madrl_h
   return MADRL_OK;
 }
 
-template <typename real>
-static int hw_upload_sensors(madrl_hostage* h) {
-  const int K = h->cfg.n_sensors;
-  real* tab = new (std::nothrow) real[2 * (size_t)K];
-  if (!tab) return MADRL_ENOMEM;
-  const double step = (2.0 * M_PI - 0.0) / (double)K;   // hw:27-29
-  for (int k = 0; k < K; ++k) {
-    const double a = (double)k * step + 0.0;
-    tab[k] = (real)cos(a);
-    tab[K + k] = (real)sin(a);
-  }
-  cudaError_t e = cudaMemcpy(h->state + h->lay.sensors, tab, sizeof(real) * 2 * K, cudaMemcpyHostToDevice);
-  delete[] tab;
-  MADRL_CUDA_CHECK(e);
-  return MADRL_OK;
-}
-
 extern "C" int madrl_hostage_create(const madrl_hostage_config* c, void* state_dev, madrl_hostage** out) {
   MADRL_REQUIRE(out != nullptr, "out is NULL");
   madrl_hostage_layout lay;
@@ -501,20 +478,8 @@ extern "C" int madrl_hostage_create(const madrl_hostage_config* c, void* state_d
   madrl_hostage* h = new (std::nothrow) madrl_hostage();
   if (!h) return MADRL_ENOMEM;
   h->cfg = *c; h->lay = lay;
-  h->warps_per_block = 0; h->blocks_per_sm = 0;
-  cudaError_t e = cudaGetDevice(&h->device);
-  if (e != cudaSuccess) { set_error("cudaGetDevice: %s", cudaGetErrorString(e)); delete h; return MADRL_ECUDA; }
-  h->sms = sm_count(h->device);
-  if (h->sms <= 0) { delete h; return MADRL_ECUDA; }
-  if (state_dev) { h->state = (char*)state_dev; h->owns_state = false; }
-  else {
-    e = cudaMalloc((void**)&h->state, lay.total_bytes);
-    if (e != cudaSuccess) { set_error("cudaMalloc(%zu): %s", lay.total_bytes, cudaGetErrorString(e)); delete h; return MADRL_ENOMEM; }
-    h->owns_state = true;
-  }
-  e = cudaMemset(h->state, 0, lay.total_bytes);
-  if (e != cudaSuccess) { set_error("cudaMemset: %s", cudaGetErrorString(e)); madrl_hostage_destroy(h); return MADRL_ECUDA; }
-  rc = c->fp64 ? hw_upload_sensors<double>(h) : hw_upload_sensors<float>(h);
+  rc = core_init(h, state_dev, lay.total_bytes);
+  if (!rc) rc = upload_sensor_table(h->state + lay.sensors, c->n_sensors, c->fp64);
   if (rc) { madrl_hostage_destroy(h); return rc; }
   *out = h;
   return MADRL_OK;
@@ -522,8 +487,7 @@ extern "C" int madrl_hostage_create(const madrl_hostage_config* c, void* state_d
 
 extern "C" int madrl_hostage_destroy(madrl_hostage* h) {
   if (!h) return MADRL_OK;
-  if (h->owns_state && h->state) cudaFree(h->state);
-  h->pipe.destroy();
+  core_release(h);
   delete h;
   return MADRL_OK;
 }
@@ -533,47 +497,20 @@ extern "C" void* madrl_hostage_state_ptr(madrl_hostage* h) { return h ? h->state
 extern "C" int madrl_hostage_seed(madrl_hostage* h, uint64_t seed, void* stream) {
   MADRL_REQUIRE(h != nullptr, "handle is NULL");
   h->cfg.seed = seed;
-  MADRL_CUDA_CHECK(cudaMemsetAsync(h->state + h->lay.rng_counter, 0, 8 * (size_t)h->cfg.n_envs, (cudaStream_t)stream));
-  return MADRL_OK;
+  return core_clear_counters(h, h->lay.rng_counter, h->cfg.n_envs, stream);
 }
 
 extern "C" int madrl_hostage_set_terminal_obs(madrl_hostage* h, void* term_obs_dev) {
-  MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  h->term_obs = term_obs_dev;
-  return MADRL_OK;
+  return core_set_terminal_obs(h, term_obs_dev);
 }
 
 extern "C" int madrl_hostage_set_launch(madrl_hostage* h, int warps_per_block, int blocks_per_sm) {
-  MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  MADRL_REQUIRE(warps_per_block >= 0 && warps_per_block <= 4, "warps_per_block must be in [0,4]");
-  MADRL_REQUIRE(blocks_per_sm >= 0 && blocks_per_sm <= 32, "blocks_per_sm must be in [0,32]");
-  h->warps_per_block = warps_per_block; h->blocks_per_sm = blocks_per_sm;
-  return MADRL_OK;
-}
-
-template <typename real>
-static real hw_exact_sq_threshold(double thr_d) {
-  const real thr = (real)thr_d;
-  real t = thr * thr;
-  const real up = (real)INFINITY, dn = -(real)INFINITY;
-  while (std::sqrt(t) <= thr) t = std::nextafter(t, up);
-  while (std::sqrt(t) > thr) t = std::nextafter(t, dn);
-  return t;
+  return core_set_launch(h, warps_per_block, blocks_per_sm);
 }
 
 template <typename real, int OPL, int KCH, int KC>
 static int hw_launch_inst(madrl_hostage* h, const HWParams<real>& p, cudaStream_t stream) {
-  const auto kfn = hw_kernel<real, OPL, KCH, KC>;
-  int resident = 0;
-  MADRL_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kfn, 32, 0));
-  if (resident < 1) resident = 1;
-  if (h->blocks_per_sm > 0 && h->blocks_per_sm < resident) resident = h->blocks_per_sm;
-  int grid = p.E;
-  if (grid > h->sms * resident) grid = h->sms * resident;
-  MADRL_LAUNCH(kfn, grid, 32, 0, stream, p);
-  g_launches.fetch_add(1);
-  MADRL_CUDA_CHECK(cudaGetLastError());
-  return MADRL_OK;
+  return launch_persistent(h, hw_kernel<real, OPL, KCH, KC>, p.E, 0, stream, p);
 }
 
 template <typename real>
@@ -591,10 +528,10 @@ static int hw_launch(madrl_hostage* h, int mode, int T, const void* actions, voi
   p.r_r2 = (real)(r * r);
   p.range = (real)c.sensor_range;
   p.cull2 = (real)((c.sensor_range * c.sensor_range + r * r) * (1.0 + 1e-4) + 1e-12);
-  p.coll2_c = hw_exact_sq_threshold<real>(r + r);
-  p.coll2_h = hw_exact_sq_threshold<real>(r + r * 2);
-  p.coll2_bomb = hw_exact_sq_threshold<real>(r + c.bomb_radius);
-  p.coll2_key = hw_exact_sq_threshold<real>(r + c.key_radius);
+  p.coll2_c = exact_sq_threshold<real>(r + r);
+  p.coll2_h = exact_sq_threshold<real>(r + r * 2);
+  p.coll2_bomb = exact_sq_threshold<real>(r + c.bomb_radius);
+  p.coll2_key = exact_sq_threshold<real>(r + c.key_radius);
   p.gate_lo = (real)(0.5 + r);
   p.key_x = (real)c.key_x; p.key_y = (real)c.key_y;
   p.bad_speed = (real)c.bad_speed; p.action_scale = (real)c.action_scale;
@@ -654,42 +591,21 @@ extern "C" int madrl_hostage_step(madrl_hostage* h, const void* actions_dev, voi
 
 extern "C" int madrl_hostage_reset_host(madrl_hostage* h, const uint8_t* mask_host, void* obs_host) {
   MADRL_REQUIRE(h != nullptr && obs_host != nullptr, "handle/obs is NULL");
-  const size_t E = h->cfg.n_envs, rb = h->lay.real_bytes;
-  const size_t obs_b = E * h->cfg.n_good * h->lay.obs_dim * rb, mask_off = align_up(obs_b, 256);
-  int rc = h->pipe.ensure(mask_off + E);
-  if (rc) return rc;
-  char* st = (char*)h->pipe.stage;
-  uint8_t* mask_dev = nullptr;
-  if (mask_host) {
-    mask_dev = (uint8_t*)(st + mask_off);
-    MADRL_CUDA_CHECK(cudaMemcpyAsync(mask_dev, mask_host, E, cudaMemcpyHostToDevice, 0));
-    MADRL_CUDA_CHECK(cudaMemcpyAsync(st, obs_host, obs_b, cudaMemcpyHostToDevice, 0));
-  }
-  rc = madrl_hostage_reset(h, mask_dev, st, nullptr);
-  if (rc) return rc;
-  MADRL_CUDA_CHECK(cudaMemcpyAsync(obs_host, st, obs_b, cudaMemcpyDeviceToHost, 0));
-  MADRL_CUDA_CHECK(cudaStreamSynchronize(0));
-  return MADRL_OK;
+  const size_t E = h->cfg.n_envs;
+  return core_reset_host(h, E, E * h->cfg.n_good * h->lay.obs_dim * h->lay.real_bytes, mask_host, obs_host,
+                         [&](uint8_t* mask_dev, char* obs_dev) { return madrl_hostage_reset(h, mask_dev, obs_dev, nullptr); });
 }
 
 extern "C" int madrl_hostage_rollout_host2(madrl_hostage* h, int T, const void* actions_host, void* obs_host,
                                            void* rew_host, uint8_t* done_host, int32_t* info_host,
                                            int auto_reset, int flags) {
   MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  MADRL_REQUIRE(T >= 1, "T must be >= 1");
-  MADRL_REQUIRE(actions_host && obs_host && rew_host && done_host && info_host, "NULL trajectory buffer");
-  MADRL_REQUIRE((flags & ~MADRL_HOST_OBS_LAST) == 0, "unknown flags %d", flags);
   const size_t E = h->cfg.n_envs, Nr = h->cfg.n_good, rb = h->lay.real_bytes;
   const StepBytes sb = {E * Nr * 2 * rb, E * Nr * h->lay.obs_dim * rb, E * Nr * rb, E, E * 2 * 4};
-  void* const keep = h->term_obs;    // chunk-relative offsets: the side tensor is a device-API feature
-  h->term_obs = nullptr;
-  const int rc_ = host_rollout(h->pipe, T, sb, actions_host, obs_host, rew_host, done_host, info_host,
-                      flags & MADRL_HOST_OBS_LAST,
-                      [&](int, int Tc, char* a, char* o, char* r, char* d, char* i, cudaStream_t st) {
-                        return madrl_hostage_rollout(h, Tc, a, o, r, (uint8_t*)d, (int32_t*)i, auto_reset, st);
-                      });
-  h->term_obs = keep;
-  return rc_;
+  return core_rollout_host(h, T, sb, actions_host, obs_host, rew_host, done_host, info_host, flags,
+                           [&](int, int Tc, char* a, char* o, char* r, char* d, char* i, cudaStream_t st) {
+                             return madrl_hostage_rollout(h, Tc, a, o, r, (uint8_t*)d, (int32_t*)i, auto_reset, st);
+                           });
 }
 
 extern "C" int madrl_hostage_rollout_host(madrl_hostage* h, int T, const void* actions_host, void* obs_host,

@@ -500,15 +500,9 @@ __global__ void __launch_bounds__(32, 28) pe_kernel(const __grid_constant__ PEPa
 // =================================================================================================
 using namespace madrl;
 
-struct madrl_pursuit {
+struct madrl_pursuit : EnvCore {
   madrl_pursuit_config cfg;
   madrl_pursuit_layout lay;
-  char* state;
-  bool owns_state;
-  int device, sms;
-  int warps_per_block, blocks_per_sm;
-  madrl::HostPipe pipe;   // staging + streams of the host-buffer entry points (lazily created)
-  void* term_obs;         // madrl_pursuit_set_terminal_obs (NULL = off)
 };
 
 static int pe_validate(const madrl_pursuit_config* c) {
@@ -566,20 +560,8 @@ extern "C" int madrl_pursuit_create(const madrl_pursuit_config* c, const int32_t
   madrl_pursuit* h = new (std::nothrow) madrl_pursuit();
   if (!h) return MADRL_ENOMEM;
   h->cfg = *c; h->lay = lay;
-  h->warps_per_block = 0; h->blocks_per_sm = 0;
-  cudaError_t e = cudaGetDevice(&h->device);
-  if (e != cudaSuccess) { set_error("cudaGetDevice: %s", cudaGetErrorString(e)); delete h; return MADRL_ECUDA; }
-  h->sms = sm_count(h->device);
-  if (h->sms <= 0) { delete h; return MADRL_ECUDA; }
-  if (state_dev) { h->state = (char*)state_dev; h->owns_state = false; }
-  else {
-    e = cudaMalloc((void**)&h->state, lay.total_bytes);
-    if (e != cudaSuccess) { set_error("cudaMalloc(%zu): %s", lay.total_bytes, cudaGetErrorString(e)); delete h; return MADRL_ENOMEM; }
-    h->owns_state = true;
-  }
-  e = cudaMemset(h->state, 0, lay.total_bytes);   // agents start at (0,0), local_obs zeroed (pe:119, au:22)
-  if (e != cudaSuccess) { set_error("cudaMemset: %s", cudaGetErrorString(e)); madrl_pursuit_destroy(h); return MADRL_ECUDA; }
-  // constant tables
+  rc = core_init(h, state_dev, lay.total_bytes);   // zeroed: agents start at (0,0), local_obs zeroed (pe:119, au:22)
+  if (rc) { madrl_pursuit_destroy(h); return rc; }
   // constant table: per map the EMPTY bordered cell grid exactly as the kernel keeps it in shared memory (a rebuild
   // is a straight copy).  Word of map cell (x, y) at [(x + pad) ysP + (y + pad)]:
   //   bit 0      building (da:110-113)
@@ -613,7 +595,7 @@ extern "C" int madrl_pursuit_create(const madrl_pursuit_config* c, const int32_t
   const float lnf = (float)c->layer_norm;
   for (int k = 0; k < 256; ++k) lut[k] = (float)k / lnf;            // float32 |count| / layer_norm (pe:438)
   for (int i = 0; i < 32; ++i) idv[i] = (float)((double)i / (double)c->n_pursuers);   // pe:445
-  e = cudaMemcpy(h->state + lay.maps, m8, 4 * nm * ncellP, cudaMemcpyHostToDevice);
+  cudaError_t e = cudaMemcpy(h->state + lay.maps, m8, 4 * nm * ncellP, cudaMemcpyHostToDevice);
   delete[] m8;
   if (e == cudaSuccess) e = cudaMemcpy(h->state + lay.lut, lut, sizeof(lut), cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaMemcpy(h->state + lay.idv, idv, sizeof(idv), cudaMemcpyHostToDevice);
@@ -625,8 +607,7 @@ extern "C" int madrl_pursuit_create(const madrl_pursuit_config* c, const int32_t
 
 extern "C" int madrl_pursuit_destroy(madrl_pursuit* h) {
   if (!h) return MADRL_OK;
-  if (h->owns_state && h->state) cudaFree(h->state);
-  h->pipe.destroy();
+  core_release(h);
   delete h;
   return MADRL_OK;
 }
@@ -636,22 +617,15 @@ extern "C" void* madrl_pursuit_state_ptr(madrl_pursuit* h) { return h ? h->state
 extern "C" int madrl_pursuit_seed(madrl_pursuit* h, uint64_t seed, void* stream) {
   MADRL_REQUIRE(h != nullptr, "handle is NULL");
   h->cfg.seed = seed;
-  MADRL_CUDA_CHECK(cudaMemsetAsync(h->state + h->lay.rng_counter, 0, 8 * (size_t)h->cfg.n_envs, (cudaStream_t)stream));
-  return MADRL_OK;
+  return core_clear_counters(h, h->lay.rng_counter, h->cfg.n_envs, stream);
 }
 
 extern "C" int madrl_pursuit_set_terminal_obs(madrl_pursuit* h, void* term_obs_dev) {
-  MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  h->term_obs = term_obs_dev;
-  return MADRL_OK;
+  return core_set_terminal_obs(h, term_obs_dev);
 }
 
 extern "C" int madrl_pursuit_set_launch(madrl_pursuit* h, int warps_per_block, int blocks_per_sm) {
-  MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  MADRL_REQUIRE(warps_per_block >= 0 && warps_per_block <= 4, "warps_per_block must be in [0,4]");
-  MADRL_REQUIRE(blocks_per_sm >= 0 && blocks_per_sm <= 32, "blocks_per_sm must be in [0,32]");
-  h->warps_per_block = warps_per_block; h->blocks_per_sm = blocks_per_sm;
-  return MADRL_OK;
+  return core_set_launch(h, warps_per_block, blocks_per_sm);
 }
 
 extern "C" int madrl_pursuit_set_params(madrl_pursuit* h, double catchr, double constraint_window) {
@@ -688,20 +662,8 @@ void pe_policy_table(int R, int c2, uint8_t* lut) {
 template <int EPL, int CPL, int RC, bool POLICY, bool FLAT>
 static int pe_launch_inst3(madrl_pursuit* h, PEParams& p, cudaStream_t stream) {
   const size_t smem = 1024 + (size_t)p.smem_per_warp;   // block LUT + per-warp regions
-  const auto kfn = pe_kernel<EPL, CPL, RC, POLICY, FLAT>;
   MADRL_REQUIRE(smem <= 200 * 1024, "map too large for shared memory (%zu B per block)", smem);
-  if (smem > 48 * 1024)
-    MADRL_CUDA_CHECK(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int resident = 0;
-  MADRL_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kfn, 32, smem));
-  if (resident < 1) resident = 1;
-  if (h->blocks_per_sm > 0 && h->blocks_per_sm < resident) resident = h->blocks_per_sm;
-  int grid = p.E;
-  if (grid > h->sms * resident) grid = h->sms * resident;
-  MADRL_LAUNCH(kfn, grid, 32, smem, stream, p);
-  g_launches.fetch_add(1);
-  MADRL_CUDA_CHECK(cudaGetLastError());
-  return MADRL_OK;
+  return launch_persistent(h, pe_kernel<EPL, CPL, RC, POLICY, FLAT>, p.E, smem, stream, p);
 }
 
 template <int EPL, int CPL, int RC, bool POLICY>
@@ -795,42 +757,21 @@ extern "C" int madrl_pursuit_step(madrl_pursuit* h, const int32_t* actions_dev, 
 extern "C" int madrl_pursuit_reset_host(madrl_pursuit* h, const uint8_t* mask_host, float* obs_host) {
   MADRL_REQUIRE(h != nullptr && obs_host != nullptr, "handle/obs is NULL");
   const size_t E = h->cfg.n_envs;
-  const size_t obs_b = E * h->cfg.n_pursuers * h->lay.obs_dim * 4, mask_off = align_up(obs_b, 256);
-  int rc = h->pipe.ensure(mask_off + E);
-  if (rc) return rc;
-  char* st = (char*)h->pipe.stage;
-  uint8_t* mask_dev = nullptr;
-  if (mask_host) {
-    mask_dev = (uint8_t*)(st + mask_off);
-    MADRL_CUDA_CHECK(cudaMemcpyAsync(mask_dev, mask_host, E, cudaMemcpyHostToDevice, 0));
-    MADRL_CUDA_CHECK(cudaMemcpyAsync(st, obs_host, obs_b, cudaMemcpyHostToDevice, 0));
-  }
-  rc = madrl_pursuit_reset(h, mask_dev, (float*)st, nullptr);
-  if (rc) return rc;
-  MADRL_CUDA_CHECK(cudaMemcpyAsync(obs_host, st, obs_b, cudaMemcpyDeviceToHost, 0));
-  MADRL_CUDA_CHECK(cudaStreamSynchronize(0));
-  return MADRL_OK;
+  return core_reset_host(h, E, E * h->cfg.n_pursuers * h->lay.obs_dim * 4, mask_host, obs_host,
+                         [&](uint8_t* mask_dev, char* obs_dev) { return madrl_pursuit_reset(h, mask_dev, (float*)obs_dev, nullptr); });
 }
 
 extern "C" int madrl_pursuit_rollout_host2(madrl_pursuit* h, int T, const int32_t* actions_host, float* obs_host,
                                            float* rew_host, uint8_t* done_host, int32_t* info_host, int auto_reset,
                                            int flags) {
   MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  MADRL_REQUIRE(T >= 1, "T must be >= 1");
-  MADRL_REQUIRE(actions_host && obs_host && rew_host && done_host && info_host, "NULL trajectory buffer");
-  MADRL_REQUIRE((flags & ~MADRL_HOST_OBS_LAST) == 0, "unknown flags %d", flags);
   const size_t E = h->cfg.n_envs, Np = h->cfg.n_pursuers;
   const StepBytes sb = {E * Np * 4, E * Np * h->lay.obs_dim * 4, E * Np * 4, E, E * 4};
-  void* const keep = h->term_obs;    // chunk-relative offsets: the side tensor is a device-API feature
-  h->term_obs = nullptr;
-  const int rc_ = host_rollout(h->pipe, T, sb, actions_host, obs_host, rew_host, done_host, info_host,
-                      flags & MADRL_HOST_OBS_LAST,
-                      [&](int, int Tc, char* a, char* o, char* r, char* d, char* i, cudaStream_t st) {
-                        return madrl_pursuit_rollout(h, Tc, (const int32_t*)a, (float*)o, (float*)r, (uint8_t*)d,
-                                                     (int32_t*)i, auto_reset, st);
-                      });
-  h->term_obs = keep;
-  return rc_;
+  return core_rollout_host(h, T, sb, actions_host, obs_host, rew_host, done_host, info_host, flags,
+                           [&](int, int Tc, char* a, char* o, char* r, char* d, char* i, cudaStream_t st) {
+                             return madrl_pursuit_rollout(h, Tc, (const int32_t*)a, (float*)o, (float*)r, (uint8_t*)d,
+                                                          (int32_t*)i, auto_reset, st);
+                           });
 }
 
 extern "C" int madrl_pursuit_rollout_host(madrl_pursuit* h, int T, const int32_t* actions_host, float* obs_host,

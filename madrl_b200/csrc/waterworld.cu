@@ -624,15 +624,9 @@ ww_kernel(const __grid_constant__ WWParams<real> p) {
 // =================================================================================================
 using namespace madrl;
 
-struct madrl_ww {
+struct madrl_ww : EnvCore {
   madrl_ww_config cfg;
   madrl_ww_layout lay;
-  char* state;
-  bool owns_state;
-  int device, sms;
-  int warps_per_block, blocks_per_sm;
-  madrl::HostPipe pipe;   // staging + streams of the host-buffer entry points (lazily created)
-  void* term_obs;         // madrl_ww_set_terminal_obs (NULL = off)
   // peer gather buffers (multi-GPU fused exchange); n_peers == 0: disabled
   int n_peers, peer_rank, peer_tmax;
   void* peer_rew[8];
@@ -676,24 +670,6 @@ extern "C" int madrl_ww_state_layout(const madrl_ww_config* c, madrl_ww_layout* 
   return MADRL_OK;
 }
 
-template <typename real>
-static int ww_upload_sensors(madrl_ww* h) {
-  const int K = h->cfg.n_sensors;
-  real* tab = new (std::nothrow) real[2 * (size_t)K];
-  if (!tab) return MADRL_ENOMEM;
-  // ww:29-31  angles = linspace(0, 2pi, K+1)[:-1]
-  const double step = (2.0 * M_PI - 0.0) / (double)K;
-  for (int k = 0; k < K; ++k) {
-    const double a = (double)k * step + 0.0;
-    tab[k] = (real)cos(a);
-    tab[K + k] = (real)sin(a);
-  }
-  cudaError_t e = cudaMemcpy(h->state + h->lay.sensors, tab, sizeof(real) * 2 * K, cudaMemcpyHostToDevice);
-  delete[] tab;
-  MADRL_CUDA_CHECK(e);
-  return MADRL_OK;
-}
-
 extern "C" int madrl_ww_create(const madrl_ww_config* c, void* state_dev, madrl_ww** out) {
   MADRL_REQUIRE(out != nullptr, "out is NULL");
   madrl_ww_layout lay;
@@ -703,24 +679,9 @@ extern "C" int madrl_ww_create(const madrl_ww_config* c, void* state_dev, madrl_
   if (!h) return MADRL_ENOMEM;
   h->cfg = *c;
   h->lay = lay;
-  h->warps_per_block = 0;
-  h->blocks_per_sm = 0;
   h->n_peers = 0; h->peer_rank = 0; h->peer_tmax = 0;
-  cudaError_t e = cudaGetDevice(&h->device);
-  if (e != cudaSuccess) { set_error("cudaGetDevice: %s", cudaGetErrorString(e)); delete h; return MADRL_ECUDA; }
-  h->sms = sm_count(h->device);
-  if (h->sms <= 0) { delete h; return MADRL_ECUDA; }
-  if (state_dev) {
-    h->state = (char*)state_dev;
-    h->owns_state = false;
-  } else {
-    e = cudaMalloc((void**)&h->state, lay.total_bytes);
-    if (e != cudaSuccess) { set_error("cudaMalloc(%zu): %s", lay.total_bytes, cudaGetErrorString(e)); delete h; return MADRL_ENOMEM; }
-    h->owns_state = true;
-  }
-  e = cudaMemset(h->state, 0, lay.total_bytes);
-  if (e != cudaSuccess) { set_error("cudaMemset: %s", cudaGetErrorString(e)); madrl_ww_destroy(h); return MADRL_ECUDA; }
-  rc = c->fp64 ? ww_upload_sensors<double>(h) : ww_upload_sensors<float>(h);
+  rc = core_init(h, state_dev, lay.total_bytes);
+  if (!rc) rc = upload_sensor_table(h->state + lay.sensors, c->n_sensors, c->fp64);
   if (rc) { madrl_ww_destroy(h); return rc; }
   *out = h;
   return MADRL_OK;
@@ -728,8 +689,7 @@ extern "C" int madrl_ww_create(const madrl_ww_config* c, void* state_dev, madrl_
 
 extern "C" int madrl_ww_destroy(madrl_ww* h) {
   if (!h) return MADRL_OK;
-  if (h->owns_state && h->state) cudaFree(h->state);
-  h->pipe.destroy();
+  core_release(h);
   delete h;
   return MADRL_OK;
 }
@@ -739,9 +699,7 @@ extern "C" void* madrl_ww_state_ptr(madrl_ww* h) { return h ? h->state : nullptr
 extern "C" int madrl_ww_seed(madrl_ww* h, uint64_t seed, void* stream) {
   MADRL_REQUIRE(h != nullptr, "handle is NULL");
   h->cfg.seed = seed;
-  MADRL_CUDA_CHECK(cudaMemsetAsync(h->state + h->lay.rng_counter, 0, 8 * (size_t)h->cfg.n_envs,
-                                   (cudaStream_t)stream));
-  return MADRL_OK;
+  return core_clear_counters(h, h->lay.rng_counter, h->cfg.n_envs, stream);
 }
 
 extern "C" int madrl_ww_set_peers(madrl_ww* h, int n_peers, int rank, int t_max, void* const* rew_peers,
@@ -761,49 +719,17 @@ extern "C" int madrl_ww_set_peers(madrl_ww* h, int n_peers, int rank, int t_max,
 }
 
 extern "C" int madrl_ww_set_terminal_obs(madrl_ww* h, void* term_obs_dev) {
-  MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  h->term_obs = term_obs_dev;
-  return MADRL_OK;
+  return core_set_terminal_obs(h, term_obs_dev);
 }
 
 extern "C" int madrl_ww_set_launch(madrl_ww* h, int warps_per_block, int blocks_per_sm) {
-  MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  MADRL_REQUIRE(warps_per_block >= 0 && warps_per_block <= 4, "warps_per_block must be in [0,4]");
-  MADRL_REQUIRE(blocks_per_sm >= 0 && blocks_per_sm <= 32, "blocks_per_sm must be in [0,32]");
-  h->warps_per_block = warps_per_block;
-  h->blocks_per_sm = blocks_per_sm;
-  return MADRL_OK;
-}
-
-// Largest representable t with correctly-rounded sqrt(t) <= thr: `sqrt(d2) <= thr` (what
-// scipy's cdist + `<=` computes in the reference) is then exactly `d2 <= t`.
-template <typename real>
-static real exact_sq_threshold(double thr_d) {
-  const real thr = (real)thr_d;
-  real t = thr * thr;
-  const real up = (real)INFINITY, dn = -(real)INFINITY;
-  while (std::sqrt(t) <= thr) t = std::nextafter(t, up);
-  while (std::sqrt(t) > thr) t = std::nextafter(t, dn);
-  return t;
+  return core_set_launch(h, warps_per_block, blocks_per_sm);
 }
 
 template <typename real, int OPL, int KCH, int KC, bool PEER, bool POLICY>
 static int ww_launch_inst2(madrl_ww* h, const WWParams<real>& p, cudaStream_t stream) {
-  const auto kfn = ww_kernel<real, OPL, KCH, KC, PEER, POLICY>;
-  int resident = 0;
   const size_t smem = OPL >= 2 ? (size_t)p.Nall * CandSlot<real>::kStride : 0;   // candidate slots
-  if (smem > 48 * 1024)
-    MADRL_CUDA_CHECK(cudaFuncSetAttribute(kfn,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  MADRL_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kfn, 32, smem));
-  if (resident < 1) resident = 1;
-  if (h->blocks_per_sm > 0 && h->blocks_per_sm < resident) resident = h->blocks_per_sm;
-  int grid = p.E;                                    // one warp (= one 32-thread block) per env ...
-  if (grid > h->sms * resident) grid = h->sms * resident;  // ... or a single persistent wave
-  MADRL_LAUNCH(kfn, grid, 32, smem, stream, p);
-  g_launches.fetch_add(1);
-  MADRL_CUDA_CHECK(cudaGetLastError());
-  return MADRL_OK;
+  return launch_persistent(h, ww_kernel<real, OPL, KCH, KC, PEER, POLICY>, p.E, smem, stream, p);
 }
 
 template <typename real, int OPL, int KCH, int KC>
@@ -931,44 +857,21 @@ extern "C" int madrl_ww_step(madrl_ww* h, const void* actions_dev, void* obs_dev
 // ---- host-buffer entry points -------------------------------------------------------------------
 extern "C" int madrl_ww_reset_host(madrl_ww* h, const uint8_t* mask_host, void* obs_host) {
   MADRL_REQUIRE(h != nullptr && obs_host != nullptr, "handle/obs is NULL");
-  const size_t E = h->cfg.n_envs, rb = h->lay.real_bytes;
-  const size_t obs_b = E * h->cfg.n_pursuers * h->lay.obs_dim * rb;
-  const size_t mask_off = align_up(obs_b, 256);
-  int rc = h->pipe.ensure(mask_off + E);
-  if (rc) return rc;
-  char* st = (char*)h->pipe.stage;
-  uint8_t* mask_dev = nullptr;
-  if (mask_host) {
-    mask_dev = (uint8_t*)(st + mask_off);
-    MADRL_CUDA_CHECK(cudaMemcpyAsync(mask_dev, mask_host, E, cudaMemcpyHostToDevice, 0));
-    // rows of unmasked envs must survive: seed the staging buffer with the caller's obs
-    MADRL_CUDA_CHECK(cudaMemcpyAsync(st, obs_host, obs_b, cudaMemcpyHostToDevice, 0));
-  }
-  rc = madrl_ww_reset(h, mask_dev, st, nullptr);
-  if (rc) return rc;
-  MADRL_CUDA_CHECK(cudaMemcpyAsync(obs_host, st, obs_b, cudaMemcpyDeviceToHost, 0));
-  MADRL_CUDA_CHECK(cudaStreamSynchronize(0));
-  return MADRL_OK;
+  const size_t E = h->cfg.n_envs;
+  return core_reset_host(h, E, E * h->cfg.n_pursuers * h->lay.obs_dim * h->lay.real_bytes, mask_host, obs_host,
+                         [&](uint8_t* mask_dev, char* obs_dev) { return madrl_ww_reset(h, mask_dev, obs_dev, nullptr); });
 }
 
 extern "C" int madrl_ww_rollout_host2(madrl_ww* h, int T, const void* actions_host, void* obs_host,
                                       void* rew_host, uint8_t* done_host, int32_t* info_host,
                                       int auto_reset, int flags) {
   MADRL_REQUIRE(h != nullptr, "handle is NULL");
-  MADRL_REQUIRE(T >= 1, "T must be >= 1");
-  MADRL_REQUIRE(actions_host && obs_host && rew_host && done_host && info_host, "NULL trajectory buffer");
-  MADRL_REQUIRE((flags & ~MADRL_HOST_OBS_LAST) == 0, "unknown flags %d", flags);
   const size_t E = h->cfg.n_envs, Np = h->cfg.n_pursuers, rb = h->lay.real_bytes;
   const StepBytes sb = {E * Np * 2 * rb, E * Np * h->lay.obs_dim * rb, E * Np * rb, E, E * 2 * 4};
-  void* const keep = h->term_obs;    // chunk-relative offsets: the side tensor is a device-API feature
-  h->term_obs = nullptr;
-  const int rc_ = host_rollout(h->pipe, T, sb, actions_host, obs_host, rew_host, done_host, info_host,
-                      flags & MADRL_HOST_OBS_LAST,
-                      [&](int, int Tc, char* a, char* o, char* r, char* d, char* i, cudaStream_t st) {
-                        return madrl_ww_rollout(h, Tc, a, o, r, (uint8_t*)d, (int32_t*)i, auto_reset, st);
-                      });
-  h->term_obs = keep;
-  return rc_;
+  return core_rollout_host(h, T, sb, actions_host, obs_host, rew_host, done_host, info_host, flags,
+                           [&](int, int Tc, char* a, char* o, char* r, char* d, char* i, cudaStream_t st) {
+                             return madrl_ww_rollout(h, Tc, a, o, r, (uint8_t*)d, (int32_t*)i, auto_reset, st);
+                           });
 }
 
 extern "C" int madrl_ww_rollout_host(madrl_ww* h, int T, const void* actions_host, void* obs_host,

@@ -3,18 +3,13 @@
 ``BatchedHostageWorld`` is the batched tensor API; ``ContinuousHostageWorld`` is the drop-in for
 ``madrl_environments.hostage.ContinuousHostageWorld`` (same constructor, hostage.py:75-79).
 """
-import ctypes as C
-
 import numpy as np
 import torch
 
 from . import _lib
+from ._engine import _BatchedEngine
 from .core import AbstractMAEnv, Agent, EzPickle
 from .spaces import Box
-
-
-def _ptr(t):
-    return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
 class CircAgent(Agent):
@@ -33,10 +28,13 @@ class CircAgent(Agent):
         return Box(low=-10, high=10, shape=(2,))
 
 
-class BatchedHostageWorld(object):
-    """E lockstep ContinuousHostageWorld instances resident in HBM (arguments: hostage.py:75-79)."""
+class BatchedHostageWorld(_BatchedEngine):
+    """E lockstep ContinuousHostageWorld instances resident in HBM (arguments: hostage.py:75-79).
+    Actions [T, E, n_good, 2]; info [T, E, 2] = (ho_saved, cr_encs)."""
 
     timestep_limit = 1000
+    _prefix, _Layout, _agents_attr = "hostage", _lib.HWLayout, "n_good"
+    _action_tail, _info_tail, _info_keys = (2,), (2,), ("ho_saved", "cr_encs")
 
     def __init__(self, n_envs, n_good, n_hostages, n_bad, n_coop_save, n_coop_avoid, radius=0.015,
                  key_loc=None, bad_speed=0.01, n_sensors=30, sensor_range=0.2, action_scale=0.01,
@@ -44,19 +42,11 @@ class BatchedHostageWorld(object):
                  bomb_reward=-5., bomb_radius=0.05, key_radius=0.0075, control_penalty=-.1,
                  reward_mech='global', addid=True, device=None, seed=0, env_id_base=0,
                  max_path_length=0, dtype=torch.float32):
-        if not torch.cuda.is_available():
-            raise _lib.EngineError("madrl_b200 needs a CUDA device (there is no CPU fallback)")
-        self._L = _lib.lib()
-        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None \
-            else torch.device(device)
-        if self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
-        self.dtype = dtype
         self.n_envs, self.n_good, self.n_hostages, self.n_bad = n_envs, n_good, n_hostages, n_bad
         self.n_sensors, self.reward_mech = n_sensors, reward_mech
         rand_key = key_loc is None
         kx, ky = (0.0, 0.0) if rand_key else [float(v) for v in np.asarray(key_loc).reshape(-1)[:2]]
-        self.cfg = _lib.HWConfig(
+        cfg = _lib.HWConfig(
             n_envs=n_envs, env_id_base=env_id_base, n_good=n_good, n_hostages=n_hostages, n_bad=n_bad,
             n_coop_save=n_coop_save, n_coop_avoid=n_coop_avoid, n_sensors=n_sensors,
             reward_global=int(reward_mech == 'global'), addid=int(bool(addid)),
@@ -67,23 +57,8 @@ class BatchedHostageWorld(object):
             encounter_reward=encounter_reward, not_saved_reward=float(not_saved_reward),
             bomb_reward=bomb_reward, bomb_radius=bomb_radius, key_radius=key_radius,
             control_penalty=control_penalty, seed=int(seed))
-        self.layout = _lib.HWLayout()
-        _lib.check(self._L.madrl_hostage_state_layout(C.byref(self.cfg), C.byref(self.layout)))
-        self.obs_dim, self.n_obj = int(self.layout.obs_dim), int(self.layout.n_obj)
-        with torch.cuda.device(self.device):
-            self._blob = torch.zeros(int(self.layout.total_bytes), dtype=torch.uint8, device=self.device)
-            h = C.c_void_p()
-            _lib.check(self._L.madrl_hostage_create(C.byref(self.cfg), _ptr(self._blob), C.byref(h)))
-        self._h = h
-
-    def __del__(self):
-        h, self._h = getattr(self, "_h", None), None
-        if h:
-            self._L.madrl_hostage_destroy(h)
-
-    def _view(self, off, dtype, shape):
-        n = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
-        return self._blob[off:off + n].view(dtype).view(*shape)
+        _BatchedEngine.__init__(self, cfg, device, dtype)
+        self.n_obj = int(self.layout.n_obj)
 
     @property
     def state(self):
@@ -97,88 +72,6 @@ class BatchedHostageWorld(object):
                     timestep=self._view(L.timestep, torch.int32, (E,)),
                     path_len=self._view(L.path_len, torch.int32, (E,)),
                     rng_counter=self._view(L.rng_counter, torch.int64, (E,)))
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def set_terminal_obs(self, term_obs):
-        """Keep the terminal observations of done steps: `term_obs` (same shape / dtype as the obs tensor
-        of the following auto-reset rollouts) receives, at the [t, e] slots where `done` is set, the
-        observation the env returned BEFORE it was reset in place (StandardizedEnv needs it,
-        madrl_environments/__init__.py:283-291).  None switches it off."""
-        if term_obs is not None:
-            assert term_obs.is_contiguous() and term_obs.device == self.device, "term_obs must be a contiguous device tensor"
-        self._term_keepalive = term_obs
-        _lib.check(self._L.madrl_hostage_set_terminal_obs(self._h, _ptr(term_obs)))
-
-    def set_launch(self, warps_per_block=0, blocks_per_sm=0):
-        _lib.check(self._L.madrl_hostage_set_launch(self._h, warps_per_block, blocks_per_sm))
-
-    def seed(self, seed=None):
-        s = 0 if seed is None else int(seed)
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_hostage_seed(self._h, s, self._stream()))
-        return [seed]
-
-    def reset(self, mask=None, out=None):
-        E, Nr, D = self.n_envs, self.n_good, self.obs_dim
-        obs = out if out is not None else torch.zeros((E, Nr, D), dtype=self.dtype, device=self.device)
-        if out is not None:
-            _lib.require_tensor(out, "out", self.dtype, (E, Nr, D), self.device)
-        if mask is not None:
-            mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_hostage_reset(self._h, _ptr(mask), _ptr(obs), self._stream()))
-        return obs
-
-    def _require_outputs(self, T, out, device):
-        """dtype / shape / contiguity / placement of caller-supplied trajectory buffers."""
-        obs, rew, done, info = out
-        E, A, D = self.n_envs, self.n_good, self.obs_dim
-        _lib.require_tensor(obs, "obs", self.dtype, (T, E, A, D), device)
-        _lib.require_tensor(rew, "rew", self.dtype, (T, E, A), device)
-        _lib.require_tensor(done, "done", torch.uint8, (T, E), device)
-        _lib.require_tensor(info, "info", torch.int32, (T, E) + (2,), device)
-        return obs, rew, done, info
-
-    def rollout(self, actions, auto_reset=True, out=None):
-        """actions [T, E, n_good, 2] -> (obs [T,E,Nr,D], rew [T,E,Nr], done [T,E] u8, info [T,E,2])."""
-        actions = actions.to(device=self.device, dtype=self.dtype).contiguous()
-        T = actions.shape[0]
-        E, Nr, D = self.n_envs, self.n_good, self.obs_dim
-        assert actions.shape == (T, E, Nr, 2), actions.shape
-        if out is None:
-            obs = torch.empty((T, E, Nr, D), dtype=self.dtype, device=self.device)
-            rew = torch.empty((T, E, Nr), dtype=self.dtype, device=self.device)
-            done = torch.empty((T, E), dtype=torch.uint8, device=self.device)
-            info = torch.empty((T, E, 2), dtype=torch.int32, device=self.device)
-        else:
-            obs, rew, done, info = self._require_outputs(T, out, self.device)
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_hostage_rollout(self._h, T, _ptr(actions), _ptr(obs), _ptr(rew),
-                                                     _ptr(done), _ptr(info), int(auto_reset), self._stream()))
-        return obs, rew, done, info
-
-    def step(self, actions, auto_reset=False):
-        a = torch.as_tensor(actions, device=self.device, dtype=self.dtype).reshape(1, self.n_envs, self.n_good, 2)
-        obs, rew, done, info = self.rollout(a, auto_reset=auto_reset)
-        return obs[0], rew[0], done[0], dict(ho_saved=info[0, :, 0], cr_encs=info[0, :, 1])
-
-    def rollout_host(self, actions, obs, rew, done, info, auto_reset=True, obs_last=False):
-        """rollout() with HOST tensors (pinned for full PCIe speed); the copies are inside the call,
-        chunked and overlapped with the compute (csrc/host_pipeline.cuh).  `obs_last=True`: only the last
-        step's observations come back (obs is [E, A, D]) -- the policy-on-device mode."""
-        T = actions.shape[0]
-        E, A, D = self.n_envs, self.n_good, self.obs_dim
-        _lib.require_tensor(actions, "actions", self.dtype, (T, E) + (self.n_good, 2), 'cpu')
-        _lib.require_tensor(obs, "obs", self.dtype, (E, A, D) if obs_last else (T, E, A, D), 'cpu')
-        _lib.require_tensor(rew, "rew", self.dtype, (T, E, A), 'cpu')
-        _lib.require_tensor(done, "done", torch.uint8, (T, E), 'cpu')
-        _lib.require_tensor(info, "info", torch.int32, (T, E) + (2,), 'cpu')
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_hostage_rollout_host2(self._h, T, _ptr(actions), _ptr(obs), _ptr(rew), _ptr(done),
-                                                      _ptr(info), int(auto_reset), 1 if obs_last else 0))
-        return obs, rew, done, info
 
 
 class ContinuousHostageWorld(AbstractMAEnv, EzPickle):

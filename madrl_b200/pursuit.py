@@ -11,12 +11,9 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._engine import _BatchedEngine, _HeuristicRollout
 from .core import AbstractMAEnv, Agent, EzPickle
 from .spaces import Box, Discrete
-
-
-def _ptr(t):
-    return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
 class DiscreteAgent(Agent):
@@ -38,33 +35,32 @@ class DiscreteAgent(Agent):
         return Discrete(5)
 
 
-class BatchedPursuitEvade(object):
+class BatchedPursuitEvade(_HeuristicRollout, _BatchedEngine):
     """E lockstep PursuitEvade instances resident in HBM.
 
     Keyword names follow pursuit_evade.py:49-148.  Evader motion uses the env's counter-based
     stream (the reference's default controller is an unseeded RandomState shared by every
     instance, utils/Controllers.py:11, so there is no reference stream to reproduce).
+    Actions int32 [T, E, Np]; obs / rew float32; info [T, E] int32 = evaders removed;
+    rollout_heuristic runs heuristics/pursuit.py:18-50 (walk towards the nearest visible evader, a
+    random move when none is visible).
     """
+
+    _prefix, _Layout, _agents_attr = "pursuit", _lib.PELayout, "n_pursuers"
+    _dtypes, _action_dtype, _info_keys = (torch.float32,), torch.int32, ("removed",)
 
     def __init__(self, n_envs, map_pool, n_evaders=1, n_pursuers=1, obs_range=3, flatten=True,
                  layer_norm=10, n_catch=2, catchr=0.01, term_pursuit=5.0, urgency_reward=0.0,
                  include_id=True, surround=True, constraint_window=1.0, sample_maps=False,
                  reward_mech='global', random_opponents=False, max_opponents=10, device=None, seed=0,
                  env_id_base=0, max_path_length=0):
-        if not torch.cuda.is_available():
-            raise _lib.EngineError("madrl_b200 needs a CUDA device (there is no CPU fallback)")
-        self._L = _lib.lib()
-        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None \
-            else torch.device(device)
-        if self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
         mp = np.ascontiguousarray(np.asarray(map_pool), dtype=np.int32)
         if mp.ndim == 2:
             mp = mp[None]
         self.map_pool = mp
         self.n_envs, self.n_pursuers, self.n_evaders = n_envs, n_pursuers, n_evaders
         self.obs_range, self.reward_mech, self.flatten = obs_range, reward_mech, bool(flatten)
-        self.cfg = _lib.PEConfig(
+        cfg = _lib.PEConfig(
             n_envs=n_envs, env_id_base=env_id_base, n_pursuers=n_pursuers, n_evaders=n_evaders,
             xs=mp.shape[1], ys=mp.shape[2], n_maps=mp.shape[0], obs_range=obs_range,
             flatten=int(bool(flatten)), n_catch=n_catch, surround=int(bool(surround)),
@@ -74,25 +70,8 @@ class BatchedPursuitEvade(object):
             layer_norm=float(layer_norm), catchr=float(catchr), term_pursuit=float(term_pursuit),
             urgency_reward=float(urgency_reward), constraint_window=float(constraint_window),
             seed=int(seed))
-        self.layout = _lib.PELayout()
-        _lib.check(self._L.madrl_pursuit_state_layout(C.byref(self.cfg), C.byref(self.layout)))
-        self.obs_dim = int(self.layout.obs_dim)
+        _BatchedEngine.__init__(self, cfg, device, torch.float32, create_args=(C.c_void_p(mp.ctypes.data),))
         self.n_agents = int(self.layout.n_agents)
-        with torch.cuda.device(self.device):
-            self._blob = torch.zeros(int(self.layout.total_bytes), dtype=torch.uint8, device=self.device)
-            h = C.c_void_p()
-            _lib.check(self._L.madrl_pursuit_create(C.byref(self.cfg), C.c_void_p(mp.ctypes.data),
-                                                    _ptr(self._blob), C.byref(h)))
-        self._h = h
-
-    def __del__(self):
-        h, self._h = getattr(self, "_h", None), None
-        if h:
-            self._L.madrl_pursuit_destroy(h)
-
-    def _view(self, off, dtype, shape):
-        n = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
-        return self._blob[off:off + n].view(dtype).view(*shape)
 
     @property
     def state(self):
@@ -105,22 +84,6 @@ class BatchedPursuitEvade(object):
                     rng_counter=self._view(L.rng_counter, torch.int64, (E,)),
                     stale=self._view(L.stale, torch.int16, (E, Np, RR)))
 
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def set_terminal_obs(self, term_obs):
-        """Keep the terminal observations of done steps: `term_obs` (same shape / dtype as the obs tensor
-        of the following auto-reset rollouts) receives, at the [t, e] slots where `done` is set, the
-        observation the env returned BEFORE it was reset in place (StandardizedEnv needs it,
-        madrl_environments/__init__.py:283-291).  None switches it off."""
-        if term_obs is not None:
-            assert term_obs.is_contiguous() and term_obs.device == self.device, "term_obs must be a contiguous device tensor"
-        self._term_keepalive = term_obs
-        _lib.check(self._L.madrl_pursuit_set_terminal_obs(self._h, _ptr(term_obs)))
-
-    def set_launch(self, warps_per_block=0, blocks_per_sm=0):
-        _lib.check(self._L.madrl_pursuit_set_launch(self._h, warps_per_block, blocks_per_sm))
-
     def set_params(self, catchr=None, constraint_window=None):
         """Curriculum updates (pursuit_evade.py:264-272)."""
         if catchr is not None:
@@ -129,100 +92,10 @@ class BatchedPursuitEvade(object):
             self.cfg.constraint_window = float(constraint_window)
         _lib.check(self._L.madrl_pursuit_set_params(self._h, self.cfg.catchr, self.cfg.constraint_window))
 
-    def seed(self, seed=None):
-        s = 0 if seed is None else int(seed)
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_pursuit_seed(self._h, s, self._stream()))
-        return [seed]
-
-    def reset(self, mask=None, out=None):
-        E, Np, D = self.n_envs, self.n_pursuers, self.obs_dim
-        obs = out if out is not None else torch.zeros((E, Np, D), dtype=torch.float32, device=self.device)
-        if out is not None:
-            _lib.require_tensor(out, "out", torch.float32, (E, Np, D), self.device)
-        if mask is not None:
-            mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_pursuit_reset(self._h, _ptr(mask), _ptr(obs), self._stream()))
-        return obs
-
-    def _require_outputs(self, T, out, device):
-        """dtype / shape / contiguity / placement of caller-supplied trajectory buffers."""
-        obs, rew, done, info = out
-        E, A, D = self.n_envs, self.n_pursuers, self.obs_dim
-        _lib.require_tensor(obs, "obs", torch.float32, (T, E, A, D), device)
-        _lib.require_tensor(rew, "rew", torch.float32, (T, E, A), device)
-        _lib.require_tensor(done, "done", torch.uint8, (T, E), device)
-        _lib.require_tensor(info, "info", torch.int32, (T, E) + (), device)
-        return obs, rew, done, info
-
-    def rollout(self, actions, auto_reset=True, out=None):
-        """actions int32 [T, E, Np] -> (obs [T,E,Np,D] f32, rew [T,E,Np] f32, done [T,E] u8,
-        removed [T,E] i32)."""
-        actions = actions.to(device=self.device, dtype=torch.int32).contiguous()
-        T = actions.shape[0]
-        E, Np, D = self.n_envs, self.n_pursuers, self.obs_dim
-        assert actions.shape == (T, E, Np), actions.shape
-        if out is None:
-            obs = torch.empty((T, E, Np, D), dtype=torch.float32, device=self.device)
-            rew = torch.empty((T, E, Np), dtype=torch.float32, device=self.device)
-            done = torch.empty((T, E), dtype=torch.uint8, device=self.device)
-            info = torch.empty((T, E), dtype=torch.int32, device=self.device)
-        else:
-            obs, rew, done, info = self._require_outputs(T, out, self.device)
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_pursuit_rollout(self._h, T, _ptr(actions), _ptr(obs), _ptr(rew),
-                                                     _ptr(done), _ptr(info), int(auto_reset), self._stream()))
-        return obs, rew, done, info
-
-    def rollout_heuristic(self, T, obs0, auto_reset=True, out=None, record_actions=True, py2_division=True,
-                          actions_out=None):
-        """T lockstep steps in one launch with the reference's hand-written policy
-        (heuristics/pursuit.py:18-50: walk towards the nearest visible evader, a random move when none is
-        visible) evaluated inside the kernel: closed loop, no action tensor, no per-step launch.
-        obs0 [E, Np, D] = the observation the first action is computed from (`reset()`'s, or `obs[-1]` of
-        the previous rollout).  `py2_division`: the window centre `xs / 2` (heuristics/pursuit.py:23) as
-        Python 2 -- the reference's language -- computes it (R // 2); False = Python 3 true division.
-        Returns (actions int32 [T,E,Np] or None, obs, rew, done, removed)."""
-        E, Np, D = self.n_envs, self.n_pursuers, self.obs_dim
-        _lib.require_tensor(obs0, "obs0", torch.float32, (E, Np, D), self.device)
-        if out is None:
-            obs = torch.empty((T, E, Np, D), dtype=torch.float32, device=self.device)
-            rew = torch.empty((T, E, Np), dtype=torch.float32, device=self.device)
-            done = torch.empty((T, E), dtype=torch.uint8, device=self.device)
-            info = torch.empty((T, E), dtype=torch.int32, device=self.device)
-        else:
-            obs, rew, done, info = self._require_outputs(T, out, self.device)
-        if actions_out is not None:   # caller-owned buffer for the actions taken (no allocation in a rollout loop)
-            act = _lib.require_tensor(actions_out, "actions_out", torch.int32, (T, E, Np), self.device)
-        else:
-            act = torch.empty((T, E, Np), dtype=torch.int32, device=self.device) if record_actions else None
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_pursuit_rollout_heuristic(
-                self._h, T, _ptr(obs0), _ptr(act), _ptr(obs), _ptr(rew), _ptr(done), _ptr(info), int(auto_reset),
-                int(bool(py2_division)), self._stream()))
-        return act, obs, rew, done, info
-
-    def step(self, actions, auto_reset=False):
-        a = torch.as_tensor(actions, device=self.device).to(torch.int32).reshape(1, self.n_envs, self.n_pursuers)
-        obs, rew, done, info = self.rollout(a, auto_reset=auto_reset)
-        return obs[0], rew[0], done[0], dict(removed=info[0])
-
-    def rollout_host(self, actions, obs, rew, done, info, auto_reset=True, obs_last=False):
-        """rollout() with HOST tensors (pinned for full PCIe speed); the copies are inside the call,
-        chunked and overlapped with the compute (csrc/host_pipeline.cuh).  `obs_last=True`: only the last
-        step's observations come back (obs is [E, A, D]) -- the policy-on-device mode."""
-        T = actions.shape[0]
-        E, A, D = self.n_envs, self.n_pursuers, self.obs_dim
-        _lib.require_tensor(actions, "actions", torch.int32, (T, E) + (self.n_pursuers,), 'cpu')
-        _lib.require_tensor(obs, "obs", torch.float32, (E, A, D) if obs_last else (T, E, A, D), 'cpu')
-        _lib.require_tensor(rew, "rew", torch.float32, (T, E, A), 'cpu')
-        _lib.require_tensor(done, "done", torch.uint8, (T, E), 'cpu')
-        _lib.require_tensor(info, "info", torch.int32, (T, E) + (), 'cpu')
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_pursuit_rollout_host2(self._h, T, _ptr(actions), _ptr(obs), _ptr(rew), _ptr(done),
-                                                      _ptr(info), int(auto_reset), 1 if obs_last else 0))
-        return obs, rew, done, info
+    def _policy_args(self, py2_division=True):
+        """`py2_division` (rollout_heuristic keyword): the window centre `xs / 2` (heuristics/pursuit.py:23)
+        as Python 2 -- the reference's language -- computes it (R // 2); False = Python 3 true division."""
+        return (int(bool(py2_division)),)
 
 
 class PursuitEvade(AbstractMAEnv, EzPickle):

@@ -13,6 +13,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._engine import _BatchedEngine, _HeuristicRollout
 from .core import AbstractMAEnv, Agent, EzPickle
 from .spaces import Box
 
@@ -37,20 +38,20 @@ class Archea(Agent):
         return Box(low=-1, high=1, shape=(2,))
 
 
-def _ptr(t):
-    return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
-
-
-class BatchedMAWaterWorld(object):
+class BatchedMAWaterWorld(_HeuristicRollout, _BatchedEngine):
     """E lockstep MAWaterWorld instances resident in HBM.
 
     Parameters mirror waterworld.py:77-81 plus the batch/engine arguments:
     ``n_envs``; ``device``; ``seed`` and ``env_id_base`` (RNG key = (seed, env_id_base + e), so a
     sharded batch reproduces the unsharded one); ``max_path_length`` (VecEnvExecutor horizon);
     ``dtype`` torch.float32 (production) or torch.float64 (verification build).
+    Actions [T, E, Np, 2]; info [T, E, 2] = (evcatches, pocatches); rollout_heuristic runs
+    heuristics/waterworld.py:11-53.
     """
 
     timestep_limit = 1000
+    _prefix, _Layout, _agents_attr = "ww", _lib.WWLayout, "n_pursuers"
+    _action_tail, _info_tail, _info_keys = (2,), (2,), ("evcatches", "pocatches")
 
     def __init__(self, n_envs, n_pursuers, n_evaders, n_coop=2, n_poison=10, radius=0.015,
                  obstacle_radius=0.2, obstacle_loc=np.array([0.5, 0.5]), ev_speed=0.01,
@@ -58,21 +59,12 @@ class BatchedMAWaterWorld(object):
                  poison_reward=-1., food_reward=1., encounter_reward=.05, control_penalty=-.5,
                  reward_mech='local', addid=True, speed_features=True, device=None, seed=0,
                  env_id_base=0, max_path_length=0, dtype=torch.float32):
-        if not torch.cuda.is_available():
-            raise _lib.EngineError("madrl_b200 needs a CUDA device (there is no CPU fallback)")
-        self._L = _lib.lib()
-        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None \
-            else torch.device(device)
-        if self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
-        self.dtype = dtype
-        assert dtype in (torch.float32, torch.float64)
         self.n_envs, self.n_pursuers, self.n_evaders, self.n_poison = n_envs, n_pursuers, n_evaders, n_poison
         self.n_sensors = n_sensors
         self.reward_mech = reward_mech
         rand_obst = obstacle_loc is None
         ox, oy = (0.0, 0.0) if rand_obst else (float(obstacle_loc[0]), float(obstacle_loc[1]))
-        self.cfg = _lib.WWConfig(
+        cfg = _lib.WWConfig(
             n_envs=n_envs, env_id_base=env_id_base, n_pursuers=n_pursuers, n_evaders=n_evaders,
             n_poison=n_poison, n_sensors=n_sensors, n_coop=n_coop,
             reward_global=int(reward_mech == 'global'), addid=int(bool(addid)),
@@ -83,26 +75,8 @@ class BatchedMAWaterWorld(object):
             sensor_range=sensor_range, action_scale=action_scale, poison_reward=poison_reward,
             food_reward=food_reward, encounter_reward=encounter_reward,
             control_penalty=control_penalty, seed=int(seed))
-        self.layout = _lib.WWLayout()
-        _lib.check(self._L.madrl_ww_state_layout(C.byref(self.cfg), C.byref(self.layout)))
-        self.obs_dim = int(self.layout.obs_dim)
+        _BatchedEngine.__init__(self, cfg, device, dtype)
         self.n_obj = int(self.layout.n_obj)
-        with torch.cuda.device(self.device):
-            self._blob = torch.zeros(int(self.layout.total_bytes), dtype=torch.uint8, device=self.device)
-            h = C.c_void_p()
-            _lib.check(self._L.madrl_ww_create(C.byref(self.cfg), _ptr(self._blob), C.byref(h)))
-        self._h = h
-        self._seed = int(seed)
-
-    def __del__(self):
-        h, self._h = getattr(self, "_h", None), None
-        if h:
-            self._L.madrl_ww_destroy(h)
-
-    # ------------------------------------------------------------------ state views
-    def _view(self, off, dtype, shape):
-        n = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
-        return self._blob[off:off + n].view(dtype).view(*shape)
 
     @property
     def state(self):
@@ -118,22 +92,6 @@ class BatchedMAWaterWorld(object):
             rng_counter=self._view(L.rng_counter, torch.int64, (E,)),
             sensors=self._view(L.sensors, dt, (2, self.n_sensors)))
 
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def set_terminal_obs(self, term_obs):
-        """Keep the terminal observations of done steps: `term_obs` (same shape / dtype as the obs tensor
-        of the following auto-reset rollouts) receives, at the [t, e] slots where `done` is set, the
-        observation the env returned BEFORE it was reset in place (StandardizedEnv needs it,
-        madrl_environments/__init__.py:283-291).  None switches it off."""
-        if term_obs is not None:
-            assert term_obs.is_contiguous() and term_obs.device == self.device, "term_obs must be a contiguous device tensor"
-        self._term_keepalive = term_obs
-        _lib.check(self._L.madrl_ww_set_terminal_obs(self._h, _ptr(term_obs)))
-
-    def set_launch(self, warps_per_block=0, blocks_per_sm=0):
-        _lib.check(self._L.madrl_ww_set_launch(self._h, warps_per_block, blocks_per_sm))
-
     def set_peers(self, rank, t_max, rew_peers, done_peers, info_peers):
         """Enable the fused exchange: `*_peers` are lists (one per DESTINATION rank) of tensors
         aliasing the destination gather buffers; this rank writes slot `rank` of each
@@ -147,101 +105,6 @@ class BatchedMAWaterWorld(object):
     def clear_peers(self):
         self._peer_keepalive = None
         _lib.check(self._L.madrl_ww_set_peers(self._h, 0, 0, 0, None, None, None))
-
-    # ------------------------------------------------------------------ env surface (batched)
-    def seed(self, seed=None):
-        self._seed = 0 if seed is None else int(seed)
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_ww_seed(self._h, self._seed, self._stream()))
-        return [seed]
-
-    def reset(self, mask=None, out=None):
-        """reset() of the masked envs (all if None) -> obs [E, Np, D]."""
-        E, Np, D = self.n_envs, self.n_pursuers, self.obs_dim
-        obs = out if out is not None else torch.zeros((E, Np, D), dtype=self.dtype, device=self.device)
-        if out is not None:
-            _lib.require_tensor(out, "out", self.dtype, (E, Np, D), self.device)
-        if mask is not None:
-            mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_ww_reset(self._h, _ptr(mask), _ptr(obs), self._stream()))
-        return obs
-
-    def _require_outputs(self, T, out, device):
-        """dtype / shape / contiguity / placement of caller-supplied trajectory buffers."""
-        obs, rew, done, info = out
-        E, A, D = self.n_envs, self.n_pursuers, self.obs_dim
-        _lib.require_tensor(obs, "obs", self.dtype, (T, E, A, D), device)
-        _lib.require_tensor(rew, "rew", self.dtype, (T, E, A), device)
-        _lib.require_tensor(done, "done", torch.uint8, (T, E), device)
-        _lib.require_tensor(info, "info", torch.int32, (T, E) + (2,), device)
-        return obs, rew, done, info
-
-    def rollout(self, actions, auto_reset=True, out=None):
-        """T lockstep steps in one kernel launch.  actions [T, E, Np, 2] ->
-        (obs [T,E,Np,D], rew [T,E,Np], done [T,E] uint8, info [T,E,2] int32)."""
-        actions = actions.to(device=self.device, dtype=self.dtype).contiguous()
-        T = actions.shape[0]
-        E, Np, D = self.n_envs, self.n_pursuers, self.obs_dim
-        assert actions.shape == (T, E, Np, 2), actions.shape
-        if out is None:
-            obs = torch.empty((T, E, Np, D), dtype=self.dtype, device=self.device)
-            rew = torch.empty((T, E, Np), dtype=self.dtype, device=self.device)
-            done = torch.empty((T, E), dtype=torch.uint8, device=self.device)
-            info = torch.empty((T, E, 2), dtype=torch.int32, device=self.device)
-        else:
-            obs, rew, done, info = self._require_outputs(T, out, self.device)
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_ww_rollout(self._h, T, _ptr(actions), _ptr(obs), _ptr(rew),
-                                                _ptr(done), _ptr(info), int(auto_reset), self._stream()))
-        return obs, rew, done, info
-
-    def rollout_heuristic(self, T, obs0, auto_reset=True, out=None, record_actions=True, actions_out=None):
-        """T lockstep steps in one launch with the reference's hand-written policy
-        (heuristics/waterworld.py:11-53) evaluated inside the kernel: closed loop, no action tensor,
-        no per-step launch.  obs0 [E, Np, D] = the observation the first action is computed from
-        (`reset()`'s, or `obs[-1]` of the previous rollout).  Returns
-        (actions [T,E,Np,2] or None, obs, rew, done, info)."""
-        E, Np, D = self.n_envs, self.n_pursuers, self.obs_dim
-        _lib.require_tensor(obs0, "obs0", self.dtype, (E, Np, D), self.device)
-        if out is None:
-            obs = torch.empty((T, E, Np, D), dtype=self.dtype, device=self.device)
-            rew = torch.empty((T, E, Np), dtype=self.dtype, device=self.device)
-            done = torch.empty((T, E), dtype=torch.uint8, device=self.device)
-            info = torch.empty((T, E, 2), dtype=torch.int32, device=self.device)
-        else:
-            obs, rew, done, info = self._require_outputs(T, out, self.device)
-        if actions_out is not None:   # caller-owned buffer for the actions taken (no allocation in a rollout loop)
-            act = _lib.require_tensor(actions_out, "actions_out", self.dtype, (T, E, Np, 2), self.device)
-        else:
-            act = torch.empty((T, E, Np, 2), dtype=self.dtype, device=self.device) if record_actions else None
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_ww_rollout_heuristic(self._h, T, _ptr(obs0), _ptr(act), _ptr(obs), _ptr(rew),
-                                                          _ptr(done), _ptr(info), int(auto_reset), self._stream()))
-        return act, obs, rew, done, info
-
-    def step(self, actions, auto_reset=False):
-        """One lockstep step.  actions [E, Np, 2] (or anything reshapeable to it)."""
-        a = torch.as_tensor(actions, device=self.device, dtype=self.dtype).reshape(
-            1, self.n_envs, self.n_pursuers, 2)
-        obs, rew, done, info = self.rollout(a, auto_reset=auto_reset)
-        return obs[0], rew[0], done[0], dict(evcatches=info[0, :, 0], pocatches=info[0, :, 1])
-
-    def rollout_host(self, actions, obs, rew, done, info, auto_reset=True, obs_last=False):
-        """rollout() with HOST tensors (pinned for full PCIe speed); the copies are inside the call,
-        chunked and overlapped with the compute (csrc/host_pipeline.cuh).  `obs_last=True`: only the last
-        step's observations come back (obs is [E, A, D]) -- the policy-on-device mode."""
-        T = actions.shape[0]
-        E, A, D = self.n_envs, self.n_pursuers, self.obs_dim
-        _lib.require_tensor(actions, "actions", self.dtype, (T, E) + (self.n_pursuers, 2), 'cpu')
-        _lib.require_tensor(obs, "obs", self.dtype, (E, A, D) if obs_last else (T, E, A, D), 'cpu')
-        _lib.require_tensor(rew, "rew", self.dtype, (T, E, A), 'cpu')
-        _lib.require_tensor(done, "done", torch.uint8, (T, E), 'cpu')
-        _lib.require_tensor(info, "info", torch.int32, (T, E) + (2,), 'cpu')
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.madrl_ww_rollout_host2(self._h, T, _ptr(actions), _ptr(obs), _ptr(rew), _ptr(done),
-                                                      _ptr(info), int(auto_reset), 1 if obs_last else 0))
-        return obs, rew, done, info
 
 
 class MAWaterWorld(AbstractMAEnv, EzPickle):

@@ -78,11 +78,13 @@ def test_masked_reset_and_seed(name):
 
 
 def test_error_codes_and_messages():
-    from madrl_b200 import BatchedMAWaterWorld, EngineError, _lib
+    from madrl_b200 import BatchedHostageWorld, BatchedMAWaterWorld, EngineError, _lib
     with pytest.raises(EngineError, match="n_pursuers"):
         BatchedMAWaterWorld(4, 40, 5)
     with pytest.raises(EngineError, match="n_sensors"):
         BatchedMAWaterWorld(4, 5, 5, n_sensors=100)
+    with pytest.raises(TypeError, match="dtype"):       # no fp16 kernel: would write 4-byte values into 2-byte rows
+        BatchedHostageWorld(4, 2, 2, 2, 1, 1, dtype=torch.float16)
     eng = BatchedMAWaterWorld(4, 5, 5)
     lib = _lib.lib()
     assert lib.madrl_ww_rollout(eng._h, 0, None, None, None, None, None, 0, None) == -1
@@ -90,3 +92,13 @@ def test_error_codes_and_messages():
     assert lib.madrl_ww_reset(None, None, None, None) == -1
     with pytest.raises(EngineError):
         eng.set_launch(warps_per_block=9)
+    # the terminal-obs side tensor is written at the [t, e] slots of every later auto-reset rollout
+    T, shape = 6, (6, 4, 5, eng.obs_dim)
+    with pytest.raises(TypeError, match="term_obs"):
+        eng.set_terminal_obs(torch.zeros(shape, dtype=torch.float64, device=eng.device))
+    eng.set_terminal_obs(torch.zeros((T - 1,) + shape[1:], dtype=torch.float32, device=eng.device))
+    eng.reset()
+    n = _lib.launch_count()
+    with pytest.raises(ValueError, match="term_obs"):
+        eng.rollout(torch.zeros(T, 4, 5, 2, device=eng.device), auto_reset=True)
+    assert _lib.launch_count() == n                      # refused before the launch
